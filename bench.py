@@ -5,7 +5,7 @@ Workload (BASELINE.json configs[1]): standalone dequant sweep Q4_0 / Q4_K / Q5_K
 Flux.1-dev Linear weight shapes, fp16 output, reference-default fp16 math.  One STEP = one pass over all 35 packed
 tensors (35 kernel launches, 1.42 G elements, 1.05 GB packed read + 2.83 GB written).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 value      algorithmic GB/s (packed bytes read + output bytes written) / device time, inputs resident in HBM
 e2e        same metric and the same 35 tensors through the plugin call (`dequantize_tensor`) with HOST buffers: pinned-host
@@ -16,6 +16,9 @@ cpu_baseline  the C oracle port of the reference algorithm on the host cores (bo
 N > 1      independent replicas (one process per GPU, torchrun), no collective on the data path; value = sum of
            units / max-over-ranks device time  ("scaling": "weak")
 --impl reference   times the reference's CPU algorithm (oracle port, all host threads) on the same 35 tensors per step
+--dump-outputs DIR   after the timed steps, writes what the last step computed as DIR/<qtype>_<N>x<K>.npy (float32): a
+           fixed, seeded sample of DUMP_SAMPLE elements of each fp16 result (flattened row-major, sample positions ascending),
+           36.7 MB in all.  The packed inputs are seeded, so two builds run with the same arguments can be compared file for file
 """
 from __future__ import annotations
 
@@ -36,6 +39,7 @@ FLUX_SHAPES = [(18432, 3072), (9216, 3072), (3072, 3072), (12288, 3072), (3072, 
 QTYPES = ["Q4_0", "Q4_K", "Q5_K", "Q6_K", "Q8_0"]
 METRIC = "standalone dequant throughput, GGUF packed -> fp16 (algorithmic GB/s = packed bytes read + output bytes written)"
 UNIT = "GB/s"
+DUMP_SAMPLE = 1 << 18      # elements per dumped tensor (35 tensors x 1 MiB of float32)
 WORKLOAD = ("configs[1]: standalone dequant sweep Q4_0/Q4_K/Q5_K/Q6_K/Q8_0 x 7 Flux.1-dev Linear shapes "
             "([18432|9216|3072|12288|21504,3072],[3072,12288|15360]), fp16 out, fp16 reference math")
 
@@ -147,6 +151,21 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons)}
 
 
+def dump_outputs(out_dir, tensors, dev):
+    """The fp16 results of the last timed step (what dequantize_tensor hands a caller), as float32 samples: the same
+    DUMP_SAMPLE flat positions of every tensor of a shape on every run (seeded), ascending."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    positions = {}
+    for t in tensors:
+        N, K = t["shape"]
+        if (N, K) not in positions:
+            rng = np.random.default_rng(N * 100003 + K)
+            positions[N, K] = torch.from_numpy(np.sort(rng.choice(N * K, size=min(N * K, DUMP_SAMPLE), replace=False))).to(dev)
+        got = t["out"].reshape(-1)[positions[N, K]].float().cpu().numpy()
+        np.save(os.path.join(out_dir, f"{t['q']}_{N}x{K}.npy"), got)
+
+
 def cpu_baseline_run(budget_s=12.0, threads=None):
     """The reference algorithm on the host: C oracle port (OpenMP, all threads) on a bounded sample of the workload:
     the [3072,3072] member of every qtype in the sweep, fp16 math, fp16 out; repeated until ~budget_s."""
@@ -194,38 +213,28 @@ def cpu_baseline_run(budget_s=12.0, threads=None):
         tot_s += med
     res["numpy_gguf_py"] = {"value": tot_bytes / tot_s / 1e9, "unit": UNIT, "cores": 1, "per_qtype": per_q,
                             "sample": f"gguf.quants.dequantize [3072,3072] -> fp32 for each of {'/'.join(QTYPES)}, median of 5 after 1 warm-up"}
-    # the reference's own torch path on CPU tensors (dequant.py::dequantize_tensor), when the reference checkout is present
-    # (this container; it does not travel to the GPU box)
-    ref_py = "/root/reference/dequant.py"
-    if os.path.exists(ref_py):
-        try:
-            import importlib.util
-            import torch
-            spec = importlib.util.spec_from_file_location("ref_dequant_bench", ref_py)
-            refdq = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(refdq)
-            per_q, tot_bytes, tot_s = {}, 0.0, 0.0
-            for q, code, raw in tensors:
-                qt = gguf.GGMLQuantizationType(code)
-                data = torch.from_numpy(raw.reshape(N, -1))
-                refdq.dequantize(data, qt, (N, K), dtype=None)
-                ts_ = []
-                for _ in range(5):
-                    t1 = time.perf_counter()
-                    refdq.dequantize(data, qt, (N, K), dtype=None)
-                    ts_.append(time.perf_counter() - t1)
-                med = float(np.median(ts_))
-                b = alg_bytes(q, N * K)
-                per_q[q] = b / med / 1e9
-                tot_bytes += b
-                tot_s += med
-            res["torch_cpu_reference"] = {"value": tot_bytes / tot_s / 1e9, "unit": UNIT, "cores": torch.get_num_threads(), "per_qtype": per_q,
-                                          "kind": "reference", "sample": "the unmodified /root/reference/dequant.py::dequantize on CPU tensors "
-                                          f"[3072,3072] for each of {'/'.join(QTYPES)}, fp16 math, median of 5 after 1 warm-up"}
-        except Exception as exc:
-            res["torch_cpu_reference"] = {"unavailable": repr(exc)[:160]}
-    else:
-        res["torch_cpu_reference"] = {"unavailable": "/root/reference is not present on this box (GPU box); see profiles/ for the container run"}
+    # the reference's own torch path on CPU tensors (dequant.py::dequantize): oracle/torch_chain.py issues the same ATen
+    # kernels and gives the same bits (tests/test_torch_chain.py pins both against the reference's stored outputs)
+    import torch
+    from oracle import torch_chain
+    per_q, tot_bytes, tot_s = {}, 0.0, 0.0
+    for q, code, raw in tensors:
+        qt = gguf.GGMLQuantizationType(code)
+        data = torch.from_numpy(raw.reshape(N, -1))
+        torch_chain.dequantize(data, qt, (N, K), dtype=None)
+        ts_ = []
+        for _ in range(5):
+            t1 = time.perf_counter()
+            torch_chain.dequantize(data, qt, (N, K), dtype=None)
+            ts_.append(time.perf_counter() - t1)
+        med = float(np.median(ts_))
+        b = alg_bytes(q, N * K)
+        per_q[q] = b / med / 1e9
+        tot_bytes += b
+        tot_s += med
+    res["torch_cpu_reference"] = {"value": tot_bytes / tot_s / 1e9, "unit": UNIT, "cores": torch.get_num_threads(), "per_qtype": per_q,
+                                  "kind": "reference", "sample": "the reference's dequant.py::dequantize torch chain (oracle/torch_chain.py) "
+                                  f"on CPU tensors [3072,3072] for each of {'/'.join(QTYPES)}, fp16 math, median of 5 after 1 warm-up"}
     return res
 
 
@@ -294,7 +303,10 @@ def main():
     ap.add_argument("--eager", action="store_true", help="time eager launches instead of replaying each step from a CUDA graph")
     ap.add_argument("--sweep-detail", action="store_true", help="also print per-(qtype,shape) GB/s lines to stderr")
     ap.add_argument("--no-flux", action="store_true", help="skip the secondary metric (Flux.1-shape Q4_K denoise step A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of what the last timed step computed to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -401,6 +413,8 @@ def main():
     torch.cuda.synchronize()
     rep.barrier()
     local_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tensors, dev)
     total_ms = rep.max_over_ranks(local_ms)
     total_bytes = rep.sum_over_ranks(float(step_bytes) * args.steps)
     value = total_bytes / (total_ms * 1e-3) / 1e9

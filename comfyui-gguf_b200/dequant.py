@@ -1,6 +1,6 @@
 """Drop-in for the reference's dequant.py: same public names, B200 kernels underneath.
 
-Reference surface mirrored (file:line in /root/reference):
+Reference surface mirrored (file:line in city96/ComfyUI-GGUF):
     is_torch_compatible / is_quantized       dequant.py:9-13
     dequantize_tensor(tensor, dtype, dequant_dtype)   dequant.py:15-28
     dequantize(data, qtype, oshape, dtype)   dequant.py:30-44

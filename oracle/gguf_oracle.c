@@ -9,7 +9,7 @@
  *
  * Parity pinning: the reference ships no golden vectors of its own (SURVEY.md
  * section 8c), so this restatement is pinned against outputs of the reference
- * itself: tests/golden/make_golden.py imports /root/reference/dequant.py
+ * itself: tests/golden/make_golden.py imports the reference's dequant.py
  * unmodified, runs it on seeded blocks and commits the results under
  * tests/golden/; tests/test_oracle.py requires bit-equality with those files and
  * with gguf-py's numpy `gguf.quants.dequantize` (the reference's fallback path,

@@ -1,11 +1,11 @@
 """The reference's torch-GPU execution path, restated for A/B timing -- TEST / BENCH INFRASTRUCTURE ONLY.
 
-/root/reference does not exist on the GPU box, so the "reference torch-GPU path" that BASELINE.json asks the
-fused kernels to beat is re-expressed here as the same chain of unfused ATen ops the reference issues per
-Linear call (dequant.py:30-44 -> dequantize_blocks_* -> `.to(dtype)` -> F.linear, ops.py:242-244), including
-its per-call creation of the small shift tensors on the device.  tests/test_torch_chain.py pins this file
-against the unmodified reference (bit-equal outputs AND the same number of materialising ATen kernels) in the
-build container.  Nothing in the product package imports it.
+The "reference torch-GPU path" that BASELINE.json asks the fused kernels to beat is re-expressed here, so that
+the project can time it without the reference installed, as the same chain of unfused ATen ops the reference
+issues per Linear call (dequant.py:30-44 -> dequantize_blocks_* -> `.to(dtype)` -> F.linear, ops.py:242-244),
+including its per-call creation of the small shift tensors on the device.  tests/test_torch_chain.py pins this
+file against outputs of the unmodified reference stored under tests/golden/ (bit-equal outputs AND the same
+number of materialising ATen kernels).  Nothing in the product package imports it.
 
 Types covered: the ones the BASELINE configs use on the GPU A/B (Q4_K, Q5_K, Q6_K, Q8_0, Q4_0, BF16).
 """

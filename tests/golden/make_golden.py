@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """Generate the committed golden vectors from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference, which does not exist on
-the GPU box):   python tests/golden/make_golden.py
+Needs a checkout of the original ComfyUI-GGUF (city96/ComfyUI-GGUF, commit
+795e45156ece) and runs on the CPU:
+
+    python tests/golden/make_golden.py REFERENCE_DIR [dequant|linear|torch_chain|surface ...]
+
+(default: all four groups; a group rewrites only its own files)
 
 What is produced (all under tests/golden/):
   dequant_<QTYPE>.npz   seeded packed blocks + the reference's own outputs of
@@ -11,12 +15,20 @@ What is produced (all under tests/golden/):
   linear_<QTYPE>_<act>.npz   x / packed W / F32 bias and the output of the
                         reference `ops.py::GGMLOps.Linear.forward` (run on CPU
                         through tests/fake_comfy)
+  torch_chain_reference.json   per (qtype, math dtype) of tests/test_torch_chain.py:
+                        dtype, SHA-256 of the bytes and a seeded sample of the
+                        bit patterns of `dequant.py::dequantize`, and the number
+                        of materialising ATen kernels it issues
+  reference_surface.json   public function / class names of dequant.py and ops.py
 
 The reference is imported by path and never copied: dequant.py via importlib,
 ops.py through a throw-away package directory of symlinks in $TMPDIR.
 """
+import ast
+import hashlib
 import importlib
 import importlib.util
+import json
 import os
 import sys
 import tempfile
@@ -27,9 +39,10 @@ import gguf
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = None      # the original checkout, from the command line
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests", "fake_comfy"))
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import oracle  # noqa: E402  (only for the seeded block generator)
 
@@ -135,8 +148,48 @@ def make_linear(refops):
         print("wrote linear", qt.name)
 
 
+def make_torch_chain(ref):
+    """What tests/test_torch_chain.py compares oracle/torch_chain.py with: the full output is pinned by its SHA-256, a
+    seeded sample of 64 bit patterns makes a mismatch readable."""
+    from test_torch_chain import MATH_DTYPES, QTYPES as CHAIN_QTYPES, Count, case_id, inputs, output_bits
+    out = {}
+    for qt, md in ((qt, md) for md in MATH_DTYPES for qt in CHAIN_QTYPES):
+        raw, shape = inputs(qt)
+        with Count() as c:
+            a = ref.dequantize(raw, qt, shape, dtype=md)
+        b = output_bits(a)
+        idx = np.sort(np.random.default_rng(0).choice(b.size, size=min(64, b.size), replace=False))
+        out[case_id(qt, md)] = {"dtype": str(a.dtype), "shape": list(a.shape), "aten_kernels": c.n,
+                                "sha256": hashlib.sha256(b.tobytes()).hexdigest(),
+                                "sample_index": idx.tolist(), "sample_bits": b[idx].tolist()}
+    with open(os.path.join(HERE, "torch_chain_reference.json"), "w") as f:       # one case per line
+        f.write("{\n" + ",\n".join(f" {json.dumps(k)}: {json.dumps(v)}" for k, v in out.items()) + "\n}\n")
+    print("wrote torch_chain_reference.json", len(out), "cases")
+
+
+def make_surface():
+    """Public top-level function / class names of the original dequant.py and ops.py (tests/test_host.py)."""
+    def public(path):
+        tree = ast.parse(open(path).read())
+        return sorted(n.name for n in tree.body if isinstance(n, (ast.FunctionDef, ast.ClassDef)) and not n.name.startswith("_"))
+    with open(os.path.join(HERE, "reference_surface.json"), "w") as f:
+        json.dump({name: public(os.path.join(REF, name)) for name in ("dequant.py", "ops.py")}, f, indent=1)
+        f.write("\n")
+    print("wrote reference_surface.json")
+
+
 if __name__ == "__main__":
+    if len(sys.argv) < 2 or not os.path.isfile(os.path.join(sys.argv[1], "dequant.py")):
+        sys.exit(__doc__)
+    REF = os.path.abspath(sys.argv[1])
+    groups = sys.argv[2:] or ["dequant", "linear", "torch_chain", "surface"]
     torch.manual_seed(0)
-    make_dequant(load_ref_dequant())
-    make_linear(load_ref_ops())
-    print("total bytes:", sum(os.path.getsize(os.path.join(HERE, f)) for f in os.listdir(HERE) if f.endswith(".npz")))
+    if "dequant" in groups:
+        make_dequant(load_ref_dequant())
+    if "linear" in groups:
+        make_linear(load_ref_ops())
+    if "torch_chain" in groups:
+        make_torch_chain(load_ref_dequant())
+    if "surface" in groups:
+        make_surface()
+    print("total bytes:", sum(os.path.getsize(os.path.join(HERE, f)) for f in os.listdir(HERE) if f.endswith((".npz", ".json"))))

@@ -22,6 +22,24 @@ def test_reference_arm_json_contract():
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_dump_outputs_is_a_seeded_float32_sample(tmp_path):
+    """--dump-outputs: one float32 file per result, the same positions on every run, in ascending order."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    big = torch.linspace(-1, 1, 1024 * 512).half().reshape(1024, 512)       # non-decreasing, so order is visible
+    small = torch.randn(8, 32).half()
+    tensors = [{"q": "Q4_K", "shape": (1024, 512), "out": big}, {"q": "Q8_0", "shape": (8, 32), "out": small}]
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), tensors, torch.device("cpu"))
+    assert sorted(os.listdir(tmp_path / "a")) == ["Q4_K_1024x512.npy", "Q8_0_8x32.npy"]
+    a, b = np.load(tmp_path / "a" / "Q4_K_1024x512.npy"), np.load(tmp_path / "b" / "Q4_K_1024x512.npy")
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_SAMPLE,) and np.array_equal(a, b)
+    assert np.all(np.diff(a) >= 0) and np.isin(a, big.float().numpy()).all()
+    assert np.array_equal(np.load(tmp_path / "a" / "Q8_0_8x32.npy"), small.float().numpy().reshape(-1))   # smaller than the sample: all
+
+
 def test_non_leader_rank_of_reference_arm_exits_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],

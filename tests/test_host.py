@@ -1,4 +1,5 @@
 """CPU tests of the host-side mirror of the reference interface (GGMLTensor / GGMLLayer / GGMLOps / loader)."""
+import json
 import os
 
 import numpy as np
@@ -8,8 +9,6 @@ import gguf
 
 import oracle
 from util import Q
-
-REF = "/root/reference"
 
 
 def _q8_tensor(pkg, N=16, K=64, seed=0):
@@ -182,17 +181,14 @@ def test_t5_key_remap(pkg):
                    "encoder.block.1.layer.1.DenseReluDense.wi_0.weight": 5}
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree only exists in the build container")
-def test_surface_matches_reference(pkg):
-    """Same public names as the reference modules for the hot-path surface (SURVEY.md 8b)."""
-    import ast
-    def public(path):
-        tree = ast.parse(open(path).read())
-        return {n.name for n in tree.body if isinstance(n, (ast.FunctionDef, ast.ClassDef)) and not n.name.startswith("_")}
-    ref_dq = public(os.path.join(REF, "dequant.py"))
+def test_surface_matches_reference(pkg, golden_dir):
+    """Same public names as the reference modules for the hot-path surface (SURVEY.md 8b).  The reference's public names
+    are stored in tests/golden/reference_surface.json (tests/golden/make_golden.py)."""
+    surface = json.load(open(os.path.join(golden_dir, "reference_surface.json")))
+    ref_dq = set(surface["dequant.py"])
     for name in ("is_torch_compatible", "is_quantized", "dequantize_tensor", "dequantize"):
         assert name in ref_dq and hasattr(pkg.dequant, name)
-    ref_ops = public(os.path.join(REF, "ops.py"))
+    ref_ops = set(surface["ops.py"])
     for name in ("GGMLTensor", "GGMLLayer", "GGMLOps", "move_patch_to_device"):
         assert name in ref_ops and hasattr(pkg.ops, name)
     for cls in ("Linear", "Conv2d", "Embedding", "LayerNorm", "GroupNorm"):

@@ -1,6 +1,9 @@
-"""CPU test (build container only): oracle/torch_chain.py reproduces the reference's torch path bit-for-bit and with
-the same number of materialising ATen kernels, so that timing it on the GPU box is a fair stand-in for the reference."""
-import importlib.util
+"""CPU test: oracle/torch_chain.py reproduces the reference's torch path bit-for-bit and with the same number of
+materialising ATen kernels, so that timing it on the GPU is a fair stand-in for the reference.  What the unmodified
+reference's dequant.py::dequantize gives on the same seeded blocks is stored in tests/golden/torch_chain_reference.json
+(tests/golden/make_golden.py)."""
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -12,9 +15,10 @@ from torch.utils._python_dispatch import TorchDispatchMode
 import oracle
 from oracle import torch_chain
 
-REF = "/root/reference/dequant.py"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "torch_chain_reference.json")
 Q = gguf.GGMLQuantizationType
-pytestmark = pytest.mark.skipif(not os.path.exists(REF), reason="reference tree only exists in the build container")
+QTYPES = [Q.Q8_0, Q.Q4_0, Q.Q4_K, Q.Q5_K, Q.Q6_K, Q.BF16]
+MATH_DTYPES = [None, torch.float32, torch.bfloat16]
 
 
 class Count(TorchDispatchMode):
@@ -32,23 +36,31 @@ class Count(TorchDispatchMode):
         return func(*args, **(kwargs or {}))
 
 
-def _ref():
-    spec = importlib.util.spec_from_file_location("ref_dequant", REF)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m
+def case_id(qt, md):
+    return f"{qt.name}-{'default' if md is None else str(md).replace('torch.', '')}"
 
 
-@pytest.mark.parametrize("qt", [Q.Q8_0, Q.Q4_0, Q.Q4_K, Q.Q5_K, Q.Q6_K, Q.BF16], ids=lambda q: q.name)
-@pytest.mark.parametrize("md", [None, torch.float32, torch.bfloat16])
-def test_chain_equals_reference(qt, md):
-    ref = _ref()
+def inputs(qt):
     bs, ts = gguf.GGML_QUANT_SIZES[qt]
-    raw = torch.from_numpy(oracle.random_blocks(int(qt), 96, seed=1)).reshape(-1)
-    shape = (96 * bs,)
-    with Count() as c_ref:
-        a = ref.dequantize(raw, qt, shape, dtype=md)
+    return torch.from_numpy(oracle.random_blocks(int(qt), 96, seed=1)).reshape(-1), (96 * bs,)
+
+
+def output_bits(t):
+    """The elements of a dequantised tensor as unsigned integers of their width (bit patterns)."""
+    b = t.contiguous().view(torch.uint8).numpy()
+    return b.view({2: np.uint16, 4: np.uint32}[t.element_size()])
+
+
+@pytest.mark.parametrize("qt", QTYPES, ids=lambda q: q.name)
+@pytest.mark.parametrize("md", MATH_DTYPES)
+def test_chain_equals_reference(qt, md):
+    want = json.load(open(GOLDEN))[case_id(qt, md)]
+    raw, shape = inputs(qt)
     with Count() as c_mine:
         b = torch_chain.dequantize(raw, qt, shape, dtype=md)
-    assert a.dtype == b.dtype and torch.equal(a.view(torch.uint8), b.view(torch.uint8))
-    assert c_ref.n == c_mine.n, (c_ref.n, c_mine.n)
+    assert str(b.dtype) == want["dtype"] and list(b.shape) == want["shape"]
+    bits = output_bits(b)
+    idx = np.array(want["sample_index"])
+    assert bits[idx].tolist() == want["sample_bits"]
+    assert hashlib.sha256(bits.tobytes()).hexdigest() == want["sha256"]
+    assert c_mine.n == want["aten_kernels"], (c_mine.n, want["aten_kernels"])
