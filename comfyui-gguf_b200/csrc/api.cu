@@ -8,6 +8,7 @@
 
 namespace ggufb200 {
 extern int g_dequant_pdl;
+extern int g_dequant_prefetch;
 extern int g_gemv2_ctas;
 int dequant_dispatch(int type, const void *packed, long long n_blocks, void *out, int out_dtype, int math_dtype, cudaStream_t st, bool stable = false);
 int unpack_dispatch(int type, const void *packed, long long n_blocks, int16_t *q, int16_t *sc, int16_t *mn, cudaStream_t st);
@@ -213,6 +214,10 @@ int ggufb200_set_tuning(int key, int value)
     }
     if (key == 2) {
         g_gemv2_ctas = value;
+        return GGUFB200_OK;
+    }
+    if (key == 3 && value >= 0 && value <= 8) {
+        g_dequant_prefetch = value;
         return GGUFB200_OK;
     }
     return GGUFB200_E_UNSUPPORTED;

@@ -25,6 +25,7 @@ namespace ggufb200 {
 constexpr int kThreads = 128;       // threads per CTA of the dequant kernel = 4096-element tiles (256: 0.929, 64: 0.80 of the copy peak on the Flux-shape sweep)
 
 int g_dequant_pdl = 1;          // programmatic dependent launch of the dequant kernel; ggufb200_set_tuning(1, 0/1)
+int g_dequant_prefetch = 1;     // L2 prefetch distance of the dequant kernel in waves (0 = off); ggufb200_set_tuning(3, n)
 
 // Store into the OUTPUT tile.  No "memory" clobber: the output tile never aliases the packed tile the unpack reads, so the
 // compiler may keep the bytes it has already loaded (the high nibbles of a 4-bit block sit in the same bytes as the low ones)
@@ -74,10 +75,11 @@ __device__ __forceinline__ void dequant_tile(const uint8_t *tile, uint8_t *otile
 }
 
 // One tile per CTA (see the file header).  flags: bit 0 = the packed pointer is 16-byte aligned (bulk copy legal),
-// bit 1 = GGUFB200_DEQUANT_SRC_STABLE.
+// bit 1 = GGUFB200_DEQUANT_SRC_STABLE.  pf_tiles > 0: once its own tile is requested, the CTA asks L2 for the packed tile
+// pf_tiles further on (one wave of resident CTAs ahead), so the CTA that later takes that slot finds its bytes in L2.
 template <class Q, int MATH, int OUT, int THREADS>
 __global__ void __launch_bounds__(THREADS) dequant_kernel(const __grid_constant__ CUtensorMap tmOut, const uint8_t *__restrict__ src,
-                                                          void *__restrict__ dst, long long n_blocks, int flags)
+                                                          void *__restrict__ dst, long long n_blocks, int flags, int pf_tiles)
 {
     constexpr int OB = OutT<OUT>::bytes;
     constexpr int TILE_ELEMS = THREADS * 32;
@@ -114,6 +116,15 @@ __global__ void __launch_bounds__(THREADS) dequant_kernel(const __grid_constant_
             uint32_t bytes = (uint32_t)((len + 15) & ~15LL);
             mbar_arrive_expect_tx(full, bytes);
             bulk_g2s(tile, src + off, bytes, full);
+            if (pf_tiles > 0) {
+                // whole 16-byte units inside the tensor only: the prefetch never reaches past its last byte
+                const long long poff = off + (long long)pf_tiles * TILE_BYTES;
+                long long plen = total_bytes - poff;
+                if (plen > TILE_BYTES) plen = TILE_BYTES;
+                plen &= ~15LL;
+                if (plen > 0)
+                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src + poff), "r"((uint32_t)plen) : "memory");
+            }
             mbar_wait(full, 0);
         }
     } else {
@@ -225,6 +236,17 @@ template <class Q, int MATH, int OUT> static int launch_dequant(const void *pack
     }
     int flags = ((reinterpret_cast<uintptr_t>(packed) & 15) == 0) ? 1 : 0;
     if (src_stable) flags |= 2;
+    // one wave = the CTAs resident on the whole GPU at once (occupancy query, once per device)
+    static int wave[64] = {};
+    const int dev = device_slot();
+    if (dev < 0) return GGUFB200_E_CUDA;
+    if (wave[dev] == 0) {
+        int per_sm = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, THREADS, SMEM) != cudaSuccess || per_sm <= 0) return GGUFB200_E_CUDA;
+        wave[dev] = per_sm * sm_count();
+    }
+    const long long pf = (long long)g_dequant_prefetch * wave[dev];
+    const int pf_tiles = pf < n_tiles ? (int)pf : 0;
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3((unsigned)n_tiles);
     cfg.blockDim = dim3(THREADS);
@@ -235,7 +257,7 @@ template <class Q, int MATH, int OUT> static int launch_dequant(const void *pack
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = g_dequant_pdl ? 1 : 0;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tmOut, reinterpret_cast<const uint8_t *>(packed), out, (long long)n_blocks, flags);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tmOut, reinterpret_cast<const uint8_t *>(packed), out, (long long)n_blocks, flags, pf_tiles);
     return e == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
 }
 

@@ -225,7 +225,8 @@ int ggufb200_linear_plan(int ggml_type, int64_t M, int64_t N, int64_t K, size_t 
 
 /* Benchmark-only launch knobs (they never change routing or results):
  * key 1 = programmatic dependent launch of the standalone dequant kernel (default 1),
- * key 2 = CTAs per SM of the small-M integer-pattern kernel (0 = planner picks).
+ * key 2 = CTAs per SM of the small-M integer-pattern kernel (0 = planner picks),
+ * key 3 = L2 prefetch distance of the standalone dequant kernel in waves of resident CTAs, 0..8 (default 1, 0 = off).
  * Refused with GGUFB200_E_UNSUPPORTED unless the environment variable GGUFB200_ALLOW_TUNING=1 is set when the
  * library is first used; every other key is refused always (route selection is per call: GGUFB200_ALGO_* | GGUFB200_FLAG_*). */
 int ggufb200_set_tuning(int key, int value);
