@@ -39,33 +39,23 @@ int repack_dispatch(int type, const void *W, long long N, long long K, void *out
 
 using namespace ggufb200;
 
+// block size (elements) and type size (bytes) of a ggml type; BF16 counts as blocks of one 2-byte element
 static bool type_geom(int t, int *bs, int *ts)
 {
-    int b = 0, s = 0;
-    switch (t) {
-    case T_Q4_0: b = 32; s = 18; break;
-    case T_Q4_1: b = 32; s = 20; break;
-    case T_Q5_0: b = 32; s = 22; break;
-    case T_Q5_1: b = 32; s = 24; break;
-    case T_Q8_0: b = 32; s = 34; break;
-    case T_Q2_K: b = 256; s = 84; break;
-    case T_Q3_K: b = 256; s = 110; break;
-    case T_Q4_K: b = 256; s = 144; break;
-    case T_Q5_K: b = 256; s = 176; break;
-    case T_Q6_K: b = 256; s = 210; break;
-    case T_IQ4_NL: b = 32; s = 18; break;
-    case T_IQ4_XS: b = 256; s = 136; break;
-    case T_BF16: b = 1; s = 2; break;
-    default: return false;
-    }
-    if (bs) *bs = b;
-    if (ts) *ts = s;
-    return true;
+    int b = 1, s = 2;
+    const bool ok = t == T_BF16 || with_block(t, false, [&](auto q) {
+        b = decltype(q)::BS;
+        s = decltype(q)::TS;
+        return true;
+    });
+    if (ok && bs) *bs = b;
+    if (ok && ts) *ts = s;
+    return ok;
 }
 
 static bool dtype_ok(int d) { return d >= 0 && d <= 2; }
 static bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-static bool fused_type(int t) { return t != T_BF16 && type_geom(t, nullptr, nullptr); }     // every block format has a fused producer
+static bool fused_type(int t) { return with_block(t, false, [](auto) { return true; }); }     // every block format has a fused producer
 
 // ------------------------------------------------------------------ device gate
 // The library contains sm_100a code only.  Checked once per device, right before the first launch on it (argument
@@ -109,17 +99,6 @@ struct Route {
     size_t ws;         // workspace bytes the route wants (0 = none)
 };
 
-// ABI flag bits -> gemm4's internal switches (1 = fast producers, 2 = 384-token items, 4 = no split-K)
-static int g4_flags(int flags)
-{
-    int f = (flags & GGUFB200_FLAG_GENERIC) ? 0 : 1;
-    if (flags & GGUFB200_FLAG_EXACT_W) f |= 16;       // hand-written producers that keep the reference's rounding sequence
-    if (flags & GGUFB200_FLAG_TILE384) f |= 2;
-    if (flags & GGUFB200_FLAG_TILE192) f |= 32;
-    if (flags & GGUFB200_FLAG_NOSPLIT) f |= 4;
-    return f;
-}
-
 static size_t fused_mma_ws(long long M, long long N, long long K, int flags)
 {
     if (flags & GGUFB200_FLAG_NOSPLIT) return 0;
@@ -130,7 +109,7 @@ static size_t fused_mma_ws(long long M, long long N, long long K, int flags)
 // `W` may be NULL (workspace query: assume a 16-byte aligned weight); ws_avail = workspace the caller supplied (SIZE_MAX in a query);
 // have_spans: the caller also holds the re-packed span-major copy of the weight (ggufb200_repack), which the TMEM-fed
 // kernel can stage for every block format and every K
-static Route pick_route(int type, const void *W, long long M, long long N, long long K, int act, int math, int algo_flags, size_t ws_avail,
+static Route pick_route(int type, const void *W, long long M, long long N, long long K, int math, int algo_flags, size_t ws_avail,
                         bool have_spans = false)
 {
     const int algo = algo_flags & GGUFB200_ALGO_MASK;
@@ -156,10 +135,9 @@ static Route pick_route(int type, const void *W, long long M, long long N, long 
     switch (r.algo) {
     case GGUFB200_ALGO_DEQUANT_MMA: r.ws = dense; break;
     case GGUFB200_ALGO_FUSED_MMA: r.ws = fusable ? fused_mma_ws(M, N, K, flags) : 0; break;
-    case GGUFB200_ALGO_FUSED_TMEM: r.ws = gemm4_workspace(M, N, K, g4_flags(flags)); break;
+    case GGUFB200_ALGO_FUSED_TMEM: r.ws = gemm4_workspace(M, N, K, flags); break;
     default: r.ws = 0;
     }
-    (void)act;
     return r;
 }
 
@@ -265,7 +243,7 @@ int ggufb200_dequant_rows(int ggml_type, const void *packed, int64_t n_table_row
 size_t ggufb200_linear_workspace_ex(int ggml_type, int64_t M, int64_t N, int64_t K, int act_dtype, int math_dtype, int algo)
 {
     if (!type_geom(ggml_type, nullptr, nullptr) || N <= 0 || K <= 0 || M <= 0) return 0;
-    return pick_route(ggml_type, nullptr, M, N, K, act_dtype, math_dtype, algo, (size_t)-1).ws;
+    return pick_route(ggml_type, nullptr, M, N, K, math_dtype, algo, (size_t)-1).ws;
 }
 
 size_t ggufb200_linear_workspace(int ggml_type, int64_t M, int64_t N, int64_t K, int act_dtype, int algo)
@@ -302,7 +280,7 @@ static int linear_impl(int ggml_type, const void *W_packed, const void *W_spans,
         algo = GGUFB200_ALGO_DEQUANT_MMA | flags;
     }
     if (W_spans && !aligned16(W_spans)) return GGUFB200_E_ALIGN;
-    const Route r = pick_route(ggml_type, W_packed, M, N, K, act_dtype, math_dtype, algo, ws_avail, W_spans != nullptr);
+    const Route r = pick_route(ggml_type, W_packed, M, N, K, math_dtype, algo, ws_avail, W_spans != nullptr);
     // the small-M kernel stores per element: it only needs 2-byte aligned Y rows; every other route moves 16-byte vectors
     const bool vec_y = r.algo != GGUFB200_ALGO_GEMV && r.algo != GGUFB200_ALGO_GEMV_FAST;
     if (!aligned16(X) || (ldx % 8) != 0) return GGUFB200_E_ALIGN;
@@ -322,20 +300,16 @@ static int linear_impl(int ggml_type, const void *W_packed, const void *W_spans,
     case GGUFB200_ALGO_GEMV_FAST:
         if (math_dtype != kF16 || (flags & GGUFB200_FLAG_EXACT_W)) return GGUFB200_E_UNSUPPORTED;
         return gemv2_dispatch(ggml_type, W_packed, N, K, X, M, ldx, act_dtype, bias, bias_dtype, Y, ldy, st, (flags & GGUFB200_FLAG_W_STABLE) != 0);
-    case GGUFB200_ALGO_FUSED_MMA: {
+    case GGUFB200_ALGO_FUSED_MMA:
         if (!fused_type(ggml_type)) return GGUFB200_E_UNSUPPORTED;
-        int f = 0;
-        if (flags & GGUFB200_FLAG_NOSPLIT) f |= 1;
-        if (flags & GGUFB200_FLAG_UNSTAGED) f |= 2;
         return gemm2_fused_dispatch(ggml_type, W_packed, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, workspace,
-                                    ws_avail, f, st);
-    }
+                                    ws_avail, flags, st);
     case GGUFB200_ALGO_FUSED_TMEM: {
         if (!fused_type(ggml_type) || math_dtype != kF16) return GGUFB200_E_UNSUPPORTED;
         long long span_stride = 0;
         if (W_spans) repack_bytes(ggml_type, N, K, nullptr, &span_stride);
         return gemm4_fused_dispatch(ggml_type, W_packed, W_spans, span_stride, N, K, X, M, ldx, act_dtype, bias, bias_dtype, Y, ldy, workspace,
-                                    ws_avail, g4_flags(flags), lora ? lora->T : nullptr, lora ? lora->ldt : 0, lora ? lora->U : nullptr, st);
+                                    ws_avail, flags, lora ? lora->T : nullptr, lora ? lora->ldt : 0, lora ? lora->U : nullptr, st);
     }
     case GGUFB200_ALGO_DEQUANT_MMA: {
         if (ws_avail < dense) return GGUFB200_E_WORKSPACE;
@@ -400,13 +374,13 @@ int ggufb200_linear_plan(int ggml_type, int64_t M, int64_t N, int64_t K, size_t 
     const int flags = algo & ~GGUFB200_ALGO_MASK;
     if ((algo & GGUFB200_ALGO_MASK) == GGUFB200_ALGO_FUSED_TMEM) {
         int spans = 1;
-        gemm4_plan_info(M, N, K, workspace_bytes, g4_flags(flags), tile_rows, k_ranges, &spans, ctas);
+        gemm4_plan_info(M, N, K, workspace_bytes, flags, tile_rows, k_ranges, &spans, ctas);
         *kblocks_per_range = 4 * spans;
         return GGUFB200_OK;
     }
     if ((algo & GGUFB200_ALGO_MASK) != GGUFB200_ALGO_FUSED_MMA) return GGUFB200_E_UNSUPPORTED;
     int accs = 1;
-    gemm2_fused_plan_info(M, N, K, workspace_bytes, (flags & GGUFB200_FLAG_NOSPLIT) ? 1 : 0, &accs, k_ranges, kblocks_per_range, ctas);
+    gemm2_fused_plan_info(M, N, K, workspace_bytes, flags, &accs, k_ranges, kblocks_per_range, ctas);
     *tile_rows = 256 * accs;
     return GGUFB200_OK;
 }

@@ -17,6 +17,8 @@
 // (gcd(TS,16) when the tile base is 16-byte aligned).  Everything here is integer work and
 // is bit-exact against oracle/gguf_oracle.c::unpack_elem and the reference.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace ggufb200 {
@@ -221,6 +223,61 @@ template <> struct Block<T_IQ4_XS> {  // dequant.py:258-285   [d][scales_h u16][
         sc = (int)(ls | (hs << 4)) - 32;
         mn = 0;
     }
+};
+
+// ---------------------------------------------------------------- host dispatch over the formats and dtypes
+// The only place that maps a ggml type code to its Block<T>: returns f(Block<T>{}) for the 12 block formats and `other`
+// for anything else (BF16, unknown codes).  A switch of direct calls, resolved at compile time: it sits on the host path of
+// every Linear call, whose cost matters at short activations.
+template <class R, class F> R with_block(int type, R other, F &&f)
+{
+    switch (type) {
+    case T_Q4_0: return f(Block<T_Q4_0>{});
+    case T_Q4_1: return f(Block<T_Q4_1>{});
+    case T_Q5_0: return f(Block<T_Q5_0>{});
+    case T_Q5_1: return f(Block<T_Q5_1>{});
+    case T_Q8_0: return f(Block<T_Q8_0>{});
+    case T_Q2_K: return f(Block<T_Q2_K>{});
+    case T_Q3_K: return f(Block<T_Q3_K>{});
+    case T_Q4_K: return f(Block<T_Q4_K>{});
+    case T_Q5_K: return f(Block<T_Q5_K>{});
+    case T_Q6_K: return f(Block<T_Q6_K>{});
+    case T_IQ4_NL: return f(Block<T_IQ4_NL>{});
+    case T_IQ4_XS: return f(Block<T_IQ4_XS>{});
+    }
+    return other;
+}
+
+template <int D> using DType = std::integral_constant<int, D>;
+
+// f(DType<d>{}) for a dtype code d in {kF16, kBF16, kF32}, GGUFB200_E_DTYPE for anything else
+template <class F> int with_dtype(int dtype, F &&f)
+{
+    switch (dtype) {
+    case kF16: return f(DType<kF16>{});
+    case kBF16: return f(DType<kBF16>{});
+    case kF32: return f(DType<kF32>{});
+    }
+    return GGUFB200_E_DTYPE;
+}
+
+// f(DType<act>{}) for an activation dtype: bf16, otherwise fp16 (callers have validated `act`)
+template <class F> int with_act(int act, F &&f)
+{
+    return act == kBF16 ? f(DType<kBF16>{}) : f(DType<kF16>{});
+}
+
+// K elements of one span, the unit in which the fused kernels stage packed weight rows
+constexpr int kSpanK = 256;
+
+template <class Q> struct SpanOf {
+    static constexpr int BYTES = (kSpanK / Q::BS) * Q::TS;      // packed bytes of one row's span
+    // Row pitch of a staged span in shared memory (and of the re-packed span-major layout, repack.cu).  A span whose byte
+    // count is a multiple of 16 keeps it (the canonical rows can then be staged by a 2-D tensor map, which writes rows
+    // densely); the others are padded to the next ODD multiple of 16: 16-byte aligned rows whose 16-byte reads at
+    // lane = row are bank-conflict free (Q2_K 84 -> 112, Q3_K 110 -> 112, IQ4_XS 136 -> 144, Q6_K 210 -> 240).
+    static constexpr int PAD16 = (BYTES + 15) / 16 * 16;
+    static constexpr int PITCH = BYTES % 16 == 0 ? BYTES : ((PAD16 / 16) % 2 == 1 ? PAD16 : PAD16 + 16);
 };
 
 // ---------------------------------------------------------------- float step shared by every consumer

@@ -261,43 +261,10 @@ template <class Q, int MATH, int OUT> static int launch_dequant(const void *pack
     return e == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
 }
 
-template <class Q, int MATH> static int dispatch_out(const void *packed, long long n_blocks, void *out, int out_dtype, bool stable, cudaStream_t st)
-{
-    switch (out_dtype) {
-    case kF16: return launch_dequant<Q, MATH, kF16>(packed, n_blocks, out, stable, st);
-    case kBF16: return launch_dequant<Q, MATH, kBF16>(packed, n_blocks, out, stable, st);
-    case kF32: return launch_dequant<Q, MATH, kF32>(packed, n_blocks, out, stable, st);
-    }
-    return GGUFB200_E_DTYPE;
-}
-
-template <class Q> static int dispatch_math(const void *packed, long long n_blocks, void *out, int out_dtype, int math_dtype, bool stable, cudaStream_t st)
-{
-    switch (math_dtype) {
-    case kF16: return dispatch_out<Q, kF16>(packed, n_blocks, out, out_dtype, stable, st);
-    case kBF16: return dispatch_out<Q, kBF16>(packed, n_blocks, out, out_dtype, stable, st);
-    case kF32: return dispatch_out<Q, kF32>(packed, n_blocks, out, out_dtype, stable, st);
-    }
-    return GGUFB200_E_DTYPE;
-}
-
 int dequant_dispatch(int type, const void *packed, long long n_blocks, void *out, int out_dtype, int math_dtype, cudaStream_t st, bool stable)
 {
     if (n_blocks == 0) return GGUFB200_OK;
-    switch (type) {
-    case T_Q4_0: return dispatch_math<Block<T_Q4_0>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q4_1: return dispatch_math<Block<T_Q4_1>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q5_0: return dispatch_math<Block<T_Q5_0>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q5_1: return dispatch_math<Block<T_Q5_1>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q8_0: return dispatch_math<Block<T_Q8_0>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q2_K: return dispatch_math<Block<T_Q2_K>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q3_K: return dispatch_math<Block<T_Q3_K>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q4_K: return dispatch_math<Block<T_Q4_K>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q5_K: return dispatch_math<Block<T_Q5_K>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_Q6_K: return dispatch_math<Block<T_Q6_K>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_IQ4_NL: return dispatch_math<Block<T_IQ4_NL>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_IQ4_XS: return dispatch_math<Block<T_IQ4_XS>>(packed, n_blocks, out, out_dtype, math_dtype, stable, st);
-    case T_BF16: {
+    if (type == T_BF16) {
         // one 8-element vector per thread, CTAs in address order (the grid-stride loop of the kernel only runs past the first
         // iteration for tensors beyond 2^31 CTAs): same reasoning as for the block formats above
         long long blocks = (n_blocks + (long long)kThreads * 8 - 1) / ((long long)kThreads * 8);
@@ -310,8 +277,13 @@ int dequant_dispatch(int type, const void *packed, long long n_blocks, void *out
         else return GGUFB200_E_DTYPE;
         return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
     }
-    }
-    return GGUFB200_E_TYPE;
+    return with_block(type, (int)GGUFB200_E_TYPE, [&](auto q) {
+        return with_dtype(math_dtype, [&](auto math) {
+            return with_dtype(out_dtype, [&](auto o) {
+                return launch_dequant<decltype(q), math.value, o.value>(packed, n_blocks, out, stable, st);
+            });
+        });
+    });
 }
 
 template <class Q> static int launch_unpack(const void *packed, long long n_blocks, int16_t *q, int16_t *sc, int16_t *mn, cudaStream_t st)
@@ -326,21 +298,7 @@ template <class Q> static int launch_unpack(const void *packed, long long n_bloc
 int unpack_dispatch(int type, const void *packed, long long n_blocks, int16_t *q, int16_t *sc, int16_t *mn, cudaStream_t st)
 {
     if (n_blocks == 0) return GGUFB200_OK;
-    switch (type) {
-    case T_Q4_0: return launch_unpack<Block<T_Q4_0>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q4_1: return launch_unpack<Block<T_Q4_1>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q5_0: return launch_unpack<Block<T_Q5_0>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q5_1: return launch_unpack<Block<T_Q5_1>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q8_0: return launch_unpack<Block<T_Q8_0>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q2_K: return launch_unpack<Block<T_Q2_K>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q3_K: return launch_unpack<Block<T_Q3_K>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q4_K: return launch_unpack<Block<T_Q4_K>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q5_K: return launch_unpack<Block<T_Q5_K>>(packed, n_blocks, q, sc, mn, st);
-    case T_Q6_K: return launch_unpack<Block<T_Q6_K>>(packed, n_blocks, q, sc, mn, st);
-    case T_IQ4_NL: return launch_unpack<Block<T_IQ4_NL>>(packed, n_blocks, q, sc, mn, st);
-    case T_IQ4_XS: return launch_unpack<Block<T_IQ4_XS>>(packed, n_blocks, q, sc, mn, st);
-    }
-    return GGUFB200_E_TYPE;
+    return with_block(type, (int)GGUFB200_E_TYPE, [&](auto b) { return launch_unpack<decltype(b)>(packed, n_blocks, q, sc, mn, st); });
 }
 
 }  // namespace ggufb200

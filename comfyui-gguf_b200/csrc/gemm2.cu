@@ -3,16 +3,16 @@
 //   Y[M,N] = X[M,K] * W[N,K]^T (+ bias)      fp16 / bf16 activations, fp32 accumulation in TMEM
 //
 // Why pairs: a single-CTA 128xN UMMA has to stream A (128x16) AND the whole B (Nx16) through one SM's shared
-// memory port for every instruction, and that port (128 B/clk) -- not the tensor pipe -- is what bounds the
-// single-CTA kernel in gemm.cu.  With cta_group::2 each SM of the pair holds 128 rows of A and only HALF of the
+// memory port for every instruction, and that port (128 B/clk) -- not the tensor pipe -- is what bounds a
+// single-CTA kernel.  With cta_group::2 each SM of the pair holds 128 rows of A and only HALF of the
 // B tile (128 of 256 rows); the hardware reads both halves, so shared-memory traffic per flop halves.
 //
 // Cluster = 2 CTAs.  Pair tile = (256*ACCS) x 256 x 64:  ACCS accumulator sets of 256 TMEM columns each, so one
-// B tile (dequantised once, in FUSED mode) feeds 2*256*ACCS flops per element.
+// B tile (dequantised once) feeds 2*256*ACCS flops per element.
 //   CTA rank c holds   A rows  m0 + a*256 + c*128 .. +128   (a < ACCS)          -> 16 KB * ACCS per stage (TMA)
-//                      B rows  n0 + c*128 .. +128                                -> 16 KB per stage
-// Warp roles per CTA (512 threads): 0 TMA producer, 1 MMA issuer (leader CTA only), 2 TMEM alloc,
-// 4-7 epilogue acc 0, 8-15 dequant producers (FUSED), 8-11 epilogue acc 1.
+//                      B rows  n0 + c*128 .. +128                                -> 16 KB per stage (dequant producers)
+// Warp roles per CTA (512 threads): 0 TMA producer, 1 MMA issuer (leader CTA only), 2 TMEM alloc, 3 relay,
+// 4-7 epilogue acc 0, 8-15 dequant producers, 8-11 epilogue acc 1.
 // Barriers live at identical offsets in both CTAs:
 //   full_a[s]  leader's copy collects the TMA bytes of BOTH CTAs (cp.async.bulk.tensor ... .cta_group::2, mbarrier
 //              operand mapped into the leader with mapa)
@@ -24,16 +24,6 @@ namespace ggufb200 {
 
 constexpr int kG2Threads = 512;
 constexpr int kG2DequantThreads = 256;
-
-constexpr int kG2Span = 256;        // K elements covered by one packed-weight staging buffer (= 4 k-blocks)
-
-// SEG = bytes of one row's packed K-span; 0 = the format cannot be staged with a 2-D tensor map (SEG % 16 != 0)
-template <class Q> struct PackedSeg {
-    static constexpr int value = ((kG2Span / Q::BS) * Q::TS) % 16 == 0 ? (kG2Span / Q::BS) * Q::TS : 0;
-};
-template <> struct PackedSeg<void> {
-    static constexpr int value = 0;
-};
 
 template <int ACCS, int SEG = 0> struct Gemm2Cfg {
     static constexpr int A_BYTES = ACCS * 128 * kG2BK * 2;   // 16 KB per accumulator set
@@ -48,7 +38,7 @@ template <int ACCS, int SEG = 0> struct Gemm2Cfg {
 };
 
 struct Gemm2Params {
-    const uint8_t *W;      // FUSED: packed rows
+    const uint8_t *W;      // packed rows
     long long row_bytes;
     long long M, N, K;
     const void *bias;
@@ -62,20 +52,19 @@ struct Gemm2Params {
     int splits;        // host side only
 };
 
-// STAGED (FUSED only): the packed rows of the CTA's B half are staged through shared memory by a 2-D TMA over the raw
-// bytes ([N, row_bytes] uint8/uint16, box = SEG bytes x 128 rows) one 256-wide K-span (4 k-blocks) at a time, double
-// buffered, so the dequant warps read shared memory instead of paying an L2 round trip per 8 elements.  tmB is then the
-// tensor map of the packed weight.
-template <class Q, int MATH, int ACT, int ACCS, bool STAGED>
+// STAGED: the packed rows of the CTA's B half are staged through shared memory by a 2-D TMA over the raw bytes
+// (make_packed_map: box = SEG bytes x 128 rows) one 256-wide K-span (4 k-blocks) at a time, double buffered, so the
+// dequant warps read shared memory instead of paying an L2 round trip per 8 elements.  tmB is then the tensor map of the
+// packed weight (unused otherwise).  The producers run the reference's fp16 sequence.
+template <class Q, int ACT, int ACCS, bool STAGED>
 __global__ void __launch_bounds__(STAGED ? 768 : kG2Threads, 1)
 gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const Gemm2Params p)
 {
-    constexpr int SEG = STAGED ? PackedSeg<Q>::value : 0;
+    constexpr int SEG = STAGED ? SpanOf<Q>::BYTES : 0;
     constexpr int DQ = STAGED ? 512 : kG2DequantThreads;      // dequant producer threads: 16 warps when the packed rows sit in smem
     using Cfg = Gemm2Cfg<ACCS, SEG>;
-    constexpr bool FUSED = !std::is_same<Q, void>::value;
     constexpr int STAGES = Cfg::STAGES;
-    static_assert(!STAGED || (FUSED && SEG > 0), "staging needs a fused format whose K-span is a multiple of 16 bytes");
+    static_assert(SEG % 16 == 0, "staging needs a format whose K-span is a multiple of 16 bytes");
 
     extern __shared__ uint8_t g2_smem_raw[];
     uint8_t *tiles = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(g2_smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -147,11 +136,10 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
                 mbar_wait(&empty[s], (uint32_t)(((i / STAGES) & 1) ^ 1));
                 uint8_t *a_dst = tiles + s * Cfg::STAGE_BYTES;
                 const uint32_t bar = mapa_u32(smem_u32(&full_a[s]), 0);
-                if (leader) mbar_arrive_expect_tx(&full_a[s], 2 * (FUSED ? Cfg::A_BYTES : Cfg::STAGE_BYTES));
+                if (leader) mbar_arrive_expect_tx(&full_a[s], 2 * Cfg::A_BYTES);
 #pragma unroll
                 for (int a = 0; a < ACCS; ++a)
                     tma_load_2d_pair(a_dst + a * (128 * 128), &tmA, bar, kb * kG2BK, (int)(m0 + a * 256 + rank * 128));
-                if constexpr (!FUSED) tma_load_2d_pair(a_dst + Cfg::A_BYTES, &tmB, bar, kb * kG2BK, (int)(n0 + rank * 128));
             }
         }
     } else if (warp == 1) {
@@ -162,7 +150,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
                 const int s = kb % STAGES;
                 const uint32_t par = (uint32_t)((kb / STAGES) & 1);
                 mbar_wait_cluster(&full_a[s], par);
-                if constexpr (FUSED) mbar_wait_cluster(&full_b2[s], par);
+                mbar_wait_cluster(&full_b2[s], par);
                 g2_fence_after();
                 const uint32_t a_addr = smem_u32(tiles + s * Cfg::STAGE_BYTES);
                 const uint32_t b_addr = a_addr + Cfg::A_BYTES;
@@ -179,74 +167,70 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
             umma_commit_pair(tmem_full);
         }
     } else if (warp == 3) {
-        // ===================== relay (FUSED): when this CTA's half of the B tile is complete, tell the leader's MMA issuer
-        if constexpr (FUSED) {
-            if (lane == 0) {
-                for (int kb = 0; kb < num_kb; ++kb) {
-                    const int s = kb % STAGES;
-                    mbar_wait(&full_b[s], (uint32_t)((kb / STAGES) & 1));
-                    mbar_arrive_cluster(mapa_u32(smem_u32(&full_b2[s]), 0));
-                }
+        // ===================== relay: when this CTA's half of the B tile is complete, tell the leader's MMA issuer
+        if (lane == 0) {
+            for (int kb = 0; kb < num_kb; ++kb) {
+                const int s = kb % STAGES;
+                mbar_wait(&full_b[s], (uint32_t)((kb / STAGES) & 1));
+                mbar_arrive_cluster(mapa_u32(smem_u32(&full_b2[s]), 0));
             }
         }
     } else if (warp >= 8) {
-        // ===================== dequant producers (FUSED): this CTA's 128 rows of the B tile
-        if constexpr (FUSED) {
-            constexpr int TPR = DQ / 128;       // threads per B row: 2 (32 elements each) or 4 (16 elements each)
-            constexpr int CPT = 8 / TPR;        // 16-byte chunks per thread and k-block
-            const int t = threadIdx.x - 256;
-            const int row = t / TPR;            // 0..127
-            const int half = t % TPR;           // which part of the 64-wide k-block
-            const long long n = n0 + rank * 128 + row;
-            const bool valid = n < p.N;
-            const uint8_t *wrow = p.W + (valid ? n : 0) * p.row_bytes;
-            constexpr int GROUP = GroupOf<Q>::value;
-            for (int i = 0; i < num_kb; ++i) {
-                const int kb = kb0 + i;
-                const int s = i % STAGES;
-                if constexpr (STAGED) {
-                    if ((i & 3) == 0) mbar_wait(&full_p[(i >> 2) & 1], (uint32_t)((i >> 3) & 1));
-                }
-                mbar_wait(&empty[s], (uint32_t)(((i / STAGES) & 1) ^ 1));
-                const uint32_t b_row = smem_u32(tiles + s * Cfg::STAGE_BYTES + Cfg::A_BYTES) + row * 128;
-                if (valid || STAGED) {   // STAGED: rows past N were zero-filled by the TMA and dequantise to 0
-                    const long long k = (long long)kb * kG2BK + half * (CPT * 8);
-                    const int kin = STAGED ? (int)(k & (kG2Span - 1)) : 0;   // position inside the staged span
-                    const uint8_t *blk = STAGED ? packed + ((i >> 2) & 1) * Cfg::PACKED_BYTES + row * SEG + (kin / Q::BS) * Q::TS
-                                                : wrow + (k / Q::BS) * Q::TS;
-                    const int e0 = (int)(k % Q::BS);
-                    if constexpr (STAGED && CPT == 2 && MATH == kF16 && Fast16<Q, ACT>::available) {
-                        uint32_t o[8];
-                        Fast16<Q, ACT>::run(blk, e0, o);                  // hand-scheduled 16-element producer
-                        st_shared_v4(b_row + (((half * 2) ^ (row & 7)) << 4), o[0], o[1], o[2], o[3]);
-                        st_shared_v4(b_row + (((half * 2 + 1) ^ (row & 7)) << 4), o[4], o[5], o[6], o[7]);
-                    } else {
-                        const GroupScale<MATH> g0 = group_scale<Q, MATH>(blk, e0);
-                        GroupScale<MATH> g1 = g0;
-                        if constexpr (GROUP == 16 && CPT == 4) g1 = group_scale<Q, MATH>(blk, e0 + 16);
-#pragma unroll
-                        for (int c = 0; c < CPT; ++c) {
-                            typename Math<MATH>::T2 v[4];
-                            dequant_elems<Q, MATH, 8>(blk, e0 + c * 8, (GROUP == 16 && c >= 2) ? g1 : g0, v);
-                            const int chunk = half * CPT + c;
-                            st_shared_v4(b_row + ((chunk ^ (row & 7)) << 4), pack16<ACT, MATH>(v[0]), pack16<ACT, MATH>(v[1]),
-                                         pack16<ACT, MATH>(v[2]), pack16<ACT, MATH>(v[3]));
-                        }
-                    }
+        // ===================== dequant producers: this CTA's 128 rows of the B tile
+        constexpr int TPR = DQ / 128;       // threads per B row: 2 (32 elements each) or 4 (16 elements each)
+        constexpr int CPT = 8 / TPR;        // 16-byte chunks per thread and k-block
+        const int t = threadIdx.x - 256;
+        const int row = t / TPR;            // 0..127
+        const int half = t % TPR;           // which part of the 64-wide k-block
+        const long long n = n0 + rank * 128 + row;
+        const bool valid = n < p.N;
+        const uint8_t *wrow = p.W + (valid ? n : 0) * p.row_bytes;
+        constexpr int GROUP = GroupOf<Q>::value;
+        for (int i = 0; i < num_kb; ++i) {
+            const int kb = kb0 + i;
+            const int s = i % STAGES;
+            if constexpr (STAGED) {
+                if ((i & 3) == 0) mbar_wait(&full_p[(i >> 2) & 1], (uint32_t)((i >> 3) & 1));
+            }
+            mbar_wait(&empty[s], (uint32_t)(((i / STAGES) & 1) ^ 1));
+            const uint32_t b_row = smem_u32(tiles + s * Cfg::STAGE_BYTES + Cfg::A_BYTES) + row * 128;
+            if (valid || STAGED) {   // STAGED: rows past N were zero-filled by the TMA and dequantise to 0
+                const long long k = (long long)kb * kG2BK + half * (CPT * 8);
+                const int kin = STAGED ? (int)(k & (kSpanK - 1)) : 0;   // position inside the staged span
+                const uint8_t *blk = STAGED ? packed + ((i >> 2) & 1) * Cfg::PACKED_BYTES + row * SEG + (kin / Q::BS) * Q::TS
+                                            : wrow + (k / Q::BS) * Q::TS;
+                const int e0 = (int)(k % Q::BS);
+                if constexpr (STAGED && CPT == 2 && Fast16<Q, ACT>::available) {
+                    uint32_t o[8];
+                    Fast16<Q, ACT>::run(blk, e0, o);                  // hand-scheduled 16-element producer
+                    st_shared_v4(b_row + (((half * 2) ^ (row & 7)) << 4), o[0], o[1], o[2], o[3]);
+                    st_shared_v4(b_row + (((half * 2 + 1) ^ (row & 7)) << 4), o[4], o[5], o[6], o[7]);
                 } else {
+                    const GroupScale<kF16> g0 = group_scale<Q, kF16>(blk, e0);
+                    GroupScale<kF16> g1 = g0;
+                    if constexpr (GROUP == 16 && CPT == 4) g1 = group_scale<Q, kF16>(blk, e0 + 16);
 #pragma unroll
-                    for (int c = 0; c < CPT; ++c) st_shared_v4(b_row + (((half * CPT + c) ^ (row & 7)) << 4), 0, 0, 0, 0);
-                }
-                // every lane publishes its own generic-proxy writes to the async proxy, the warp converges, and ONE lane
-                // signals the CTA-local barrier (release is cumulative over what __syncwarp ordered before it).  The
-                // cluster-scope hand-off to the MMA issuer is done by the relay warp, off the dequant warps' critical path.
-                fence_proxy_async_smem();
-                __syncwarp();
-                if (lane == 0) {
-                    mbar_arrive(&full_b[s]);
-                    if constexpr (STAGED) {
-                        if ((i & 3) == 3) mbar_arrive(&empty_p[(i >> 2) & 1]);   // done with this packed buffer
+                    for (int c = 0; c < CPT; ++c) {
+                        __half2 v[4];
+                        dequant_elems<Q, kF16, 8>(blk, e0 + c * 8, (GROUP == 16 && c >= 2) ? g1 : g0, v);
+                        const int chunk = half * CPT + c;
+                        st_shared_v4(b_row + ((chunk ^ (row & 7)) << 4), pack16<ACT, kF16>(v[0]), pack16<ACT, kF16>(v[1]),
+                                     pack16<ACT, kF16>(v[2]), pack16<ACT, kF16>(v[3]));
                     }
+                }
+            } else {
+#pragma unroll
+                for (int c = 0; c < CPT; ++c) st_shared_v4(b_row + (((half * CPT + c) ^ (row & 7)) << 4), 0, 0, 0, 0);
+            }
+            // every lane publishes its own generic-proxy writes to the async proxy, the warp converges, and ONE lane
+            // signals the CTA-local barrier (release is cumulative over what __syncwarp ordered before it).  The
+            // cluster-scope hand-off to the MMA issuer is done by the relay warp, off the dequant warps' critical path.
+            fence_proxy_async_smem();
+            __syncwarp();
+            if (lane == 0) {
+                mbar_arrive(&full_b[s]);
+                if constexpr (STAGED) {
+                    if ((i & 3) == 3) mbar_arrive(&empty_p[(i >> 2) & 1]);   // done with this packed buffer
                 }
             }
         }
@@ -352,13 +336,10 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
 }
 
 // ------------------------------------------------------------------ host side
-// Per-call switches (bits of the `flags` argument; the C ABI passes them inside `algo`, see include/ggufb200.h):
-constexpr int kG2NoSplit = 1;     // never cut the K loop into ranges
-constexpr int kG2Unstaged = 2;    // producers read the packed rows straight from global / L2 (no TMA staging)
-
 // 512-row pair tiles halve the dequant work and the X traffic per flop; fall back to 256-row tiles when the last
-// wave of 512-row tiles would leave too many SM pairs idle
-static int g2_pick_accs(long long M, long long N, bool fused = false)
+// wave of 512-row tiles would leave too many SM pairs idle.  The kernel is bound by the dequant producers, whose work per
+// flop halves with 512-row tiles (measured 1.15 vs 0.62 PFLOP/s), so a partly empty last wave is the smaller evil.
+static int g2_pick_accs(long long M, long long N)
 {
     const int sms = sm_count();
     const long long pairs = sms / 2;
@@ -368,38 +349,9 @@ static int g2_pick_accs(long long M, long long N, bool fused = false)
         return (double)tiles / (double)(waves * pairs);
     };
     if (M <= 256) return 1;
-    // fused mode is bound by the dequant producers, whose work per flop halves with 512-row tiles (measured 1.15 vs
-    // 0.62 PFLOP/s), so a partly empty last wave is the smaller evil there
-    if (fused) return eff(2) * 1.15 >= eff(1) * 0.62 ? 2 : 1;
-    return eff(2) + 0.10 >= eff(1) ? 2 : 1;
+    return eff(2) * 1.15 >= eff(1) * 0.62 ? 2 : 1;
 }
 
-// split-K finalize: Y = act(sum_s P[s] + bias), slices added in ascending order
-template <int ACT>
-__global__ void __launch_bounds__(256) g2_finalize_kernel(const float *__restrict__ P, int splits, const void *__restrict__ bias, int bias_dtype,
-                                                          uint8_t *__restrict__ Y, long long M, long long N, long long ldy)
-{
-    const long long n8 = N / 8;
-    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < M * n8; i += (long long)gridDim.x * 256) {
-        const long long m = i / n8, n = (i % n8) * 8;
-        float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        for (int sp = 0; sp < splits; ++sp) {
-            const float *src = P + ((long long)sp * M + m) * N + n;
-            const float4 a = *reinterpret_cast<const float4 *>(src), b = *reinterpret_cast<const float4 *>(src + 4);
-            v[0] += a.x; v[1] += a.y; v[2] += a.z; v[3] += a.w;
-            v[4] += b.x; v[5] += b.y; v[6] += b.z; v[7] += b.w;
-        }
-        if (bias) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) v[j] += g2_bias<ACT>(bias, bias_dtype, n + j);
-        }
-        st_global_v4(Y + (m * ldy + n) * 2, g2_pack<ACT>(v[0], v[1]), g2_pack<ACT>(v[2], v[3]), g2_pack<ACT>(v[4], v[5]), g2_pack<ACT>(v[6], v[7]));
-    }
-}
-
-// Split-K factor of the fused kernel: short activations give too few (256*ACCS x 256) tiles for the 74 SM pairs, so the K
-// loop is cut into S ranges of whole 256-wide spans, each handled by its own pair (every packed byte is still read and
-// dequantised exactly once).  Returns 1 when splitting does not apply.
 // Tiling of the fused kernel: ACCS (256 or 512 activation rows per pair) and the split-K factor.
 // Short activations give too few (256*ACCS x 256) tiles for the 74 SM pairs, so the K loop is cut into S ranges of whole
 // 256-wide spans, each handled by its own pair, which stores its fp32 partial tile into its own slice of the caller's
@@ -414,10 +366,10 @@ constexpr size_t kG2SplitWsCap = 64u << 20;   // half of the 126 MB L2
 
 static G2Plan g2_fused_plan(long long M, long long N, long long K, size_t ws_bytes, bool allow_split = true)
 {
-    G2Plan plan{g2_pick_accs(M, N, true), 1};
+    G2Plan plan{g2_pick_accs(M, N), 1};
     const size_t slice = (size_t)M * (size_t)N * 4;
     if (ws_bytes > kG2SplitWsCap) ws_bytes = kG2SplitWsCap;
-    if (slice == 0 || ws_bytes < 2 * slice || !allow_split || K % kG2Span != 0) return plan;
+    if (slice == 0 || ws_bytes < 2 * slice || !allow_split || K % kSpanK != 0) return plan;
     const int sms = sm_count();
     const long long pairs = sms / 2;
     const long long tiles_n = (N + kG2BN - 1) / kG2BN;
@@ -425,12 +377,12 @@ static G2Plan g2_fused_plan(long long M, long long N, long long K, size_t ws_byt
     if (M > 256 && tiles(2) * 2 <= pairs) plan.accs = 2;
     const long long t = tiles(plan.accs);
     if (t * 2 > pairs) return plan;   // (accs unchanged in this case)
-    const long long spans = K / kG2Span;
+    const long long spans = K / kSpanK;
     long long s = pairs / t;
     if (s > spans) s = spans;
     if (s > 16) s = 16;
     if (s > (long long)(ws_bytes / slice)) s = (long long)(ws_bytes / slice);
-    if (s < 2) return G2Plan{g2_pick_accs(M, N, true), 1};
+    if (s < 2) return G2Plan{g2_pick_accs(M, N), 1};
     const long long per = (spans + s - 1) / s;
     plan.splits = (int)((spans + per - 1) / per);
     return plan;
@@ -443,14 +395,14 @@ int gemm2_fused_splits(long long M, long long N, long long K) { return g2_fused_
 static int g2_kb_per_split(long long K, int splits)
 {
     if (splits <= 1) return (int)(K / kG2BK);
-    const int spans = (int)(K / kG2Span);
+    const int spans = (int)(K / kSpanK);
     return ((spans + splits - 1) / splits) * 4;
 }
 
 // diagnostics (ggufb200_linear_plan): the tiling the fused kernel uses for this problem and workspace size
 void gemm2_fused_plan_info(long long M, long long N, long long K, size_t ws_bytes, int flags, int *accs, int *splits, int *kb_per_split, int *ctas)
 {
-    const G2Plan plan = g2_fused_plan(M, N, K, ws_bytes, !(flags & kG2NoSplit));
+    const G2Plan plan = g2_fused_plan(M, N, K, ws_bytes, !(flags & GGUFB200_FLAG_NOSPLIT));
     const long long tiles = ((M + 256 * plan.accs - 1) / (256 * plan.accs)) * ((N + kG2BN - 1) / kG2BN);
     *accs = plan.accs;
     *splits = plan.splits;
@@ -458,11 +410,11 @@ void gemm2_fused_plan_info(long long M, long long N, long long K, size_t ws_byte
     *ctas = (int)(2 * tiles * plan.splits);
 }
 
-template <class Q, int MATH, int ACT, int ACCS, bool STAGED = false>
+template <class Q, int ACT, int ACCS, bool STAGED = false>
 static int g2_launch(const CUtensorMap &tmA, const CUtensorMap &tmB, const Gemm2Params &p, cudaStream_t st)
 {
-    using Cfg = Gemm2Cfg<ACCS, STAGED ? PackedSeg<Q>::value : 0>;
-    auto kern = gemm2_kernel<Q, MATH, ACT, ACCS, STAGED>;
+    using Cfg = Gemm2Cfg<ACCS, STAGED ? SpanOf<Q>::BYTES : 0>;
+    auto kern = gemm2_kernel<Q, ACT, ACCS, STAGED>;
     static unsigned char attr[64] = {};
     if (!ensure_dynamic_smem(kern, Cfg::SMEM, attr)) return GGUFB200_E_CUDA;
     Gemm2Params q = p;
@@ -488,27 +440,6 @@ static int g2_launch(const CUtensorMap &tmA, const CUtensorMap &tmB, const Gemm2
 
 template <class Q, int ACT>
 static int g2_fused_once(const void *W, long long N, long long K, const void *X, long long M, long long ldx, const void *bias, int bias_dtype,
-                         void *Y, long long ldy, float *partial, G2Plan plan, int flags, cudaStream_t st);
-
-template <class Q, int ACT>
-static int g2_fused_act(const void *W, long long N, long long K, const void *X, long long M, long long ldx, const void *bias, int bias_dtype,
-                        void *Y, long long ldy, void *ws, size_t ws_bytes, int flags, cudaStream_t st)
-{
-    // split-K needs room for the fp32 [splits, M, N] partial results in the caller's workspace
-    const bool ws_ok = ws && (reinterpret_cast<uintptr_t>(ws) & 15) == 0;
-    const G2Plan plan = g2_fused_plan(M, N, K, ws_ok ? ws_bytes : 0, !(flags & kG2NoSplit));
-    if (plan.splits <= 1) return g2_fused_once<Q, ACT>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, nullptr, plan, flags, st);
-    float *P = reinterpret_cast<float *>(ws);
-    int rc = g2_fused_once<Q, ACT>(W, N, K, X, M, ldx, nullptr, 0, Y, ldy, P, plan, flags, st);
-    if (rc != GGUFB200_OK) return rc;
-    long long work = M * (N / 8);
-    unsigned grid = (unsigned)((work + 255) / 256 < 148 * 8 ? (work + 255) / 256 : 148 * 8);
-    g2_finalize_kernel<ACT><<<grid, 256, 0, st>>>(P, plan.splits, bias, bias_dtype, reinterpret_cast<uint8_t *>(Y), M, N, ldy);
-    return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
-}
-
-template <class Q, int ACT>
-static int g2_fused_once(const void *W, long long N, long long K, const void *X, long long M, long long ldx, const void *bias, int bias_dtype,
                          void *Y, long long ldy, float *partial, G2Plan plan, int flags, cudaStream_t st)
 {
     CUtensorMap tmA;
@@ -522,55 +453,44 @@ static int g2_fused_once(const void *W, long long N, long long K, const void *X,
     p.bias = bias; p.bias_dtype = bias_dtype;
     p.Y = reinterpret_cast<uint8_t *>(Y); p.ldy = ldy;
     const int accs = plan.accs;
-    constexpr int SEG = PackedSeg<Q>::value;
-    if constexpr (SEG > 0) {
+    if constexpr (SpanOf<Q>::BYTES % 16 == 0) {
         // stage the packed rows through shared memory when a 2-D tensor map over the raw bytes is legal
-        if (!(flags & kG2Unstaged) && K % kG2Span == 0 && p.row_bytes % 16 == 0 && (reinterpret_cast<uintptr_t>(W) & 15) == 0) {
-            G2EncodeFn fn = g2_encode_fn();
-            if (!fn) return GGUFB200_E_CUDA;
+        if (!(flags & GGUFB200_FLAG_UNSTAGED) && K % kSpanK == 0 && packed_map_ok<Q>(W, K)) {
             CUtensorMap tmW;
-            const bool wide = SEG > 256;     // inner box extent is limited to 256 elements: use 2-byte elements
-            cuuint64_t dims[2] = {(cuuint64_t)(wide ? p.row_bytes / 2 : p.row_bytes), (cuuint64_t)N};
-            cuuint64_t strides[1] = {(cuuint64_t)p.row_bytes};
-            cuuint32_t box[2] = {(cuuint32_t)(wide ? SEG / 2 : SEG), 128u};
-            cuuint32_t estr[2] = {1, 1};
-            if (fn(&tmW, wide ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(W), dims, strides, box,
-                   estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-                return GGUFB200_E_CUDA;
-            if (accs == 2) return g2_launch<Q, kF16, ACT, 2, true>(tmA, tmW, p, st);
-            return g2_launch<Q, kF16, ACT, 1, true>(tmA, tmW, p, st);
+            if (!make_packed_map<Q>(&tmW, W, N, K)) return GGUFB200_E_CUDA;
+            if (accs == 2) return g2_launch<Q, ACT, 2, true>(tmA, tmW, p, st);
+            return g2_launch<Q, ACT, 1, true>(tmA, tmW, p, st);
         }
     }
-    if (accs == 2) return g2_launch<Q, kF16, ACT, 2>(tmA, tmA, p, st);
-    return g2_launch<Q, kF16, ACT, 1>(tmA, tmA, p, st);
+    if (accs == 2) return g2_launch<Q, ACT, 2>(tmA, tmA, p, st);
+    return g2_launch<Q, ACT, 1>(tmA, tmA, p, st);
 }
 
+template <class Q, int ACT>
+static int g2_fused_act(const void *W, long long N, long long K, const void *X, long long M, long long ldx, const void *bias, int bias_dtype,
+                        void *Y, long long ldy, void *ws, size_t ws_bytes, int flags, cudaStream_t st)
+{
+    // split-K needs room for the fp32 [splits, M, N] partial results in the caller's workspace
+    const bool ws_ok = ws && (reinterpret_cast<uintptr_t>(ws) & 15) == 0;
+    const G2Plan plan = g2_fused_plan(M, N, K, ws_ok ? ws_bytes : 0, !(flags & GGUFB200_FLAG_NOSPLIT));
+    if (plan.splits <= 1) return g2_fused_once<Q, ACT>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, nullptr, plan, flags, st);
+    float *P = reinterpret_cast<float *>(ws);
+    int rc = g2_fused_once<Q, ACT>(W, N, K, X, M, ldx, nullptr, 0, Y, ldy, P, plan, flags, st);
+    if (rc != GGUFB200_OK) return rc;
+    return splitk_finalize(P, plan.splits, bias, bias_dtype, Y, M, N, ldy, ACT, st);
+}
+
+// flags: the GGUFB200_FLAG_* bits of the call (NOSPLIT, UNSTAGED)
 int gemm2_fused_dispatch(int type, const void *W, long long N, long long K, const void *X, long long M, long long ldx, int act_dtype,
                          int math_dtype, const void *bias, int bias_dtype, void *Y, long long ldy, void *ws, size_t ws_bytes, int flags,
                          cudaStream_t st)
 {
     if (math_dtype != kF16 || K % kG2BK != 0 || N % 8 != 0) return GGUFB200_E_UNSUPPORTED;
-#define GGUFB200_G2_CASE(T)                                                                                               \
-    case T:                                                                                                               \
-        return act_dtype == kBF16 ? g2_fused_act<Block<T>, kBF16>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, ws_bytes, flags, st)  \
-                                  : g2_fused_act<Block<T>, kF16>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, ws_bytes, flags, st);
-    switch (type) {
-        GGUFB200_G2_CASE(T_Q4_0)
-        GGUFB200_G2_CASE(T_Q4_1)
-        GGUFB200_G2_CASE(T_Q5_0)
-        GGUFB200_G2_CASE(T_Q5_1)
-        GGUFB200_G2_CASE(T_Q8_0)
-        GGUFB200_G2_CASE(T_Q2_K)
-        GGUFB200_G2_CASE(T_Q3_K)
-        GGUFB200_G2_CASE(T_Q4_K)
-        GGUFB200_G2_CASE(T_Q5_K)
-        GGUFB200_G2_CASE(T_Q6_K)
-        GGUFB200_G2_CASE(T_IQ4_NL)
-        GGUFB200_G2_CASE(T_IQ4_XS)
-    }
-#undef GGUFB200_G2_CASE
-    return GGUFB200_E_UNSUPPORTED;
+    return with_block(type, (int)GGUFB200_E_UNSUPPORTED, [&](auto q) {
+        return with_act(act_dtype, [&](auto act) {
+            return g2_fused_act<decltype(q), act.value>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, ws_bytes, flags, st);
+        });
+    });
 }
 
 }  // namespace ggufb200

@@ -241,8 +241,7 @@ int gemm3_dense_dispatch(const void *W, long long N, long long K, long long ldw,
     p.M = M; p.N = N; p.K = K;
     p.bias = bias; p.bias_dtype = bias_dtype;
     p.Y = reinterpret_cast<uint8_t *>(Y); p.ldy = ldy;
-    if (narrow) return act_dtype == kBF16 ? g3_launch<kBF16, 128>(tmA, tmB, p, st) : g3_launch<kF16, 128>(tmA, tmB, p, st);
-    return act_dtype == kBF16 ? g3_launch<kBF16, 256>(tmA, tmB, p, st) : g3_launch<kF16, 256>(tmA, tmB, p, st);
+    return with_act(act_dtype, [&](auto act) { return narrow ? g3_launch<act.value, 128>(tmA, tmB, p, st) : g3_launch<act.value, 256>(tmA, tmB, p, st); });
 }
 
 }  // namespace ggufb200

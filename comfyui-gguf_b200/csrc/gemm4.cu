@@ -532,29 +532,33 @@ static G4Plan g4_plan(long long M, long long N, long long K, size_t ws_bytes, in
 
 constexpr size_t kG4SplitWsCap = 64u << 20;
 
-// flags: bit 1 (2) = force 384-token items, bit 5 (32) = force 192-token items, bit 2 (4) = no split-K
-static int g4_want_accs(int flags) { return (flags & 2) ? 2 : ((flags & 32) ? 1 : 0); }
+// item height from the ABI flags: 2 = force 384-token items (TILE384 wins over TILE192), 1 = force 192-token items, 0 = cost model
+static int g4_want_accs(int flags)
+{
+    return (flags & GGUFB200_FLAG_TILE384) ? 2 : ((flags & GGUFB200_FLAG_TILE192) ? 1 : 0);
+}
 
 size_t gemm4_workspace(long long M, long long N, long long K, int flags)
 {
-    const G4Plan pl = g4_plan(M, N, K, kG4SplitWsCap, g4_want_accs(flags), !(flags & 4));
+    const G4Plan pl = g4_plan(M, N, K, kG4SplitWsCap, g4_want_accs(flags), !(flags & GGUFB200_FLAG_NOSPLIT));
     return pl.splits > 1 ? (size_t)pl.splits * (size_t)M * (size_t)N * 4 : 0;
 }
 
 void gemm4_plan_info(long long M, long long N, long long K, size_t ws_bytes, int flags, int *tile_tokens, int *splits, int *spans_per_split, int *items)
 {
-    const G4Plan pl = g4_plan(M, N, K, ws_bytes > kG4SplitWsCap ? kG4SplitWsCap : ws_bytes, g4_want_accs(flags), !(flags & 4));
+    const G4Plan pl = g4_plan(M, N, K, ws_bytes > kG4SplitWsCap ? kG4SplitWsCap : ws_bytes, g4_want_accs(flags), !(flags & GGUFB200_FLAG_NOSPLIT));
     *tile_tokens = pl.tt * pl.accs;
     *splits = pl.splits;
     *spans_per_split = pl.spans_per_split;
     *items = pl.n_items;
 }
 
+// Split-K finalize of both fused kernels (gemm2.cu, gemm4.cu): Y = act(sum_s P[s] + bias), slices added in ascending order
+// (bit-reproducible)
 template <int ACT>
-__global__ void __launch_bounds__(256) g4_finalize_kernel(const float *__restrict__ P, int splits, const void *__restrict__ bias, int bias_dtype,
-                                                          uint8_t *__restrict__ Y, long long M, long long N, long long ldy)
+__global__ void __launch_bounds__(256) splitk_finalize_kernel(const float *__restrict__ P, int splits, const void *__restrict__ bias, int bias_dtype,
+                                                              uint8_t *__restrict__ Y, long long M, long long N, long long ldy)
 {
-    // Y = act(sum_s P[s] + bias), slices added in ascending order (bit-reproducible)
     const long long n8 = N / 8;
     for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < M * n8; i += (long long)gridDim.x * 256) {
         const long long m = i / n8, n = (i % n8) * 8;
@@ -573,6 +577,17 @@ __global__ void __launch_bounds__(256) g4_finalize_kernel(const float *__restric
     }
 }
 
+int splitk_finalize(const float *P, int splits, const void *bias, int bias_dtype, void *Y, long long M, long long N, long long ldy, int act_dtype,
+                    cudaStream_t st)
+{
+    const long long work = M * (N / 8);
+    const unsigned grid = (unsigned)((work + 255) / 256 < 148 * 8 ? (work + 255) / 256 : 148 * 8);
+    return with_act(act_dtype, [&](auto act) {
+        splitk_finalize_kernel<act.value><<<grid, 256, 0, st>>>(P, splits, bias, bias_dtype, reinterpret_cast<uint8_t *>(Y), M, N, ldy);
+        return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
+    });
+}
+
 struct G4Args {
     const void *W;             // canonical packed rows
     const void *Wspan;         // re-packed span-major layout or nullptr
@@ -586,7 +601,7 @@ struct G4Args {
     long long ldy;
     void *ws;
     size_t ws_bytes;
-    int fast, want_accs, nosplit;
+    int flags;                 // GGUFB200_FLAG_* bits of the call
     const void *loraT;         // LoRA: T = x * down^T, [M, 64] activation dtype, row stride ldt (nullptr: none)
     long long ldt;
     const void *loraU;         // LoRA: U = scale * up, fp16 [N, 64] contiguous
@@ -596,7 +611,6 @@ struct G4Args {
 template <class Q, int ACT, int TT, int ACCS, int PROD>
 static int g4_launch(const G4Args &a, const G4Plan &pl, float *partial)
 {
-    constexpr int SPAN = SpanOf<Q>::BYTES;
     using Cfg = G4Cfg<SpanOf<Q>::PITCH, TT, ACCS>;
     auto kern = gemm4_kernel<Q, ACT, TT, ACCS, PROD>;
     static unsigned char attr[64] = {};
@@ -617,20 +631,8 @@ static int g4_launch(const G4Args &a, const G4Plan &pl, float *partial)
                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
             return GGUFB200_E_CUDA;
     }
-    const long long row_bytes = a.K / Q::BS * Q::TS;
-    if (a.Wspan) {
-        tmW = tmX;   // unused by the kernel in this mode
-    } else {
-        const bool wide = SPAN > 256;     // inner box extent is limited to 256 elements: use 2-byte elements
-        cuuint64_t dims[2] = {(cuuint64_t)(wide ? row_bytes / 2 : row_bytes), (cuuint64_t)a.N};
-        cuuint64_t strides[1] = {(cuuint64_t)row_bytes};
-        cuuint32_t box[2] = {(cuuint32_t)(wide ? SPAN / 2 : SPAN), 128u};
-        cuuint32_t estr[2] = {1, 1};
-        if (fn(&tmW, wide ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(a.W), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return GGUFB200_E_CUDA;
-    }
+    if (a.Wspan) tmW = tmX;   // unused by the kernel in this mode
+    else if (!make_packed_map<Q>(&tmW, a.W, a.N, a.K)) return GGUFB200_E_CUDA;
     G4Params p{};
     p.M = a.M; p.N = a.N; p.K = a.K;
     p.bias = partial ? nullptr : a.bias;
@@ -682,78 +684,41 @@ template <class Q, int ACT> static int g4_run(const G4Args &a)
     const bool ws_ok = a.ws && (reinterpret_cast<uintptr_t>(a.ws) & 15) == 0;
     size_t wsb = ws_ok ? a.ws_bytes : 0;
     if (wsb > kG4SplitWsCap) wsb = kG4SplitWsCap;
-    const G4Plan pl = g4_plan(a.M, a.N, a.K, wsb, a.want_accs, !a.nosplit);
+    const G4Plan pl = g4_plan(a.M, a.N, a.K, wsb, g4_want_accs(a.flags), !(a.flags & GGUFB200_FLAG_NOSPLIT));
     float *partial = pl.splits > 1 ? reinterpret_cast<float *>(a.ws) : nullptr;
-    // a.fast: 0 = generic producers, 1 = hand-written + fused multiply-add, 2 = hand-written + reference sequence
+    // producers: GENERIC wins over EXACT_W; otherwise hand-written, with the reference sequence under EXACT_W, else fused multiply-add
     int rc;
-    if (a.fast == 0 || !FastProducer<Q>::fast) {
+    if ((a.flags & GGUFB200_FLAG_GENERIC) || !FastProducer<Q>::fast) {
         rc = g4_tiles<Q, ACT, 0>(a, pl, partial);
-    } else if (a.fast == 2) {
+    } else if (a.flags & GGUFB200_FLAG_EXACT_W) {
         if constexpr (FmaMatters<Q>::value) rc = g4_tiles<Q, ACT, 2>(a, pl, partial);
         else rc = g4_tiles<Q, ACT, 1>(a, pl, partial);
     } else {
         rc = g4_tiles<Q, ACT, 1>(a, pl, partial);
     }
     if (rc != GGUFB200_OK || !partial) return rc;
-    const long long work = a.M * (a.N / 8);
-    const unsigned grid = (unsigned)((work + 255) / 256 < 148 * 8 ? (work + 255) / 256 : 148 * 8);
-    g4_finalize_kernel<ACT><<<grid, 256, 0, a.st>>>(partial, pl.splits, a.bias, a.bias_dtype, reinterpret_cast<uint8_t *>(a.Y), a.M, a.N, a.ldy);
-    return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
+    return splitk_finalize(partial, pl.splits, a.bias, a.bias_dtype, a.Y, a.M, a.N, a.ldy, ACT, a.st);
 }
 
-// The canonical packed layout can be staged by a 2-D tensor map when one row's span and the row stride are multiples of 16 B
-// (every other weight needs the re-packed span-major layout of repack.cu)
-template <class Q> static bool g4_canonical_ok(const void *W, long long K)
-{
-    const long long row_bytes = K / Q::BS * Q::TS;
-    return SpanOf<Q>::BYTES % 16 == 0 && row_bytes % 16 == 0 && (reinterpret_cast<uintptr_t>(W) & 15) == 0;
-}
-
-// flags: bits 0 / 4 = producers (1: hand-written, fused multiply-add; 17: hand-written, reference sequence; 0: generic),
-// bit 1 = force 384-token items (ACCS = 2), bit 5 = force 192-token items, bit 2 = no split-K
+// flags: the GGUFB200_FLAG_* bits of the call (EXACT_W, GENERIC, TILE384, TILE192, NOSPLIT)
 int gemm4_fused_dispatch(int type, const void *W, const void *Wspan, long long span_stride, long long N, long long K, const void *X, long long M,
                          long long ldx, int act_dtype, const void *bias, int bias_dtype, void *Y, long long ldy, void *ws, size_t ws_bytes,
                          int flags, const void *loraT, long long ldt, const void *loraU, cudaStream_t st)
 {
     if (N % 8 != 0 || K % 8 != 0) return GGUFB200_E_UNSUPPORTED;
-    G4Args a{W, Wspan, span_stride, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, ws_bytes, (flags & 1) ? ((flags & 16) ? 2 : 1) : 0, (flags & 2) ? 2 : ((flags & 32) ? 1 : 0), (flags & 4) ? 1 : 0,
-             loraT, ldt, loraU, st};
-#define GGUFB200_G4_CASE(T)                                                                    \
-    case T:                                                                                    \
-        if (!Wspan && !g4_canonical_ok<Block<T>>(W, K)) return GGUFB200_E_UNSUPPORTED;         \
-        return act_dtype == kBF16 ? g4_run<Block<T>, kBF16>(a) : g4_run<Block<T>, kF16>(a);
-    switch (type) {
-        GGUFB200_G4_CASE(T_Q4_0)
-        GGUFB200_G4_CASE(T_Q4_1)
-        GGUFB200_G4_CASE(T_Q5_0)
-        GGUFB200_G4_CASE(T_Q5_1)
-        GGUFB200_G4_CASE(T_Q8_0)
-        GGUFB200_G4_CASE(T_Q2_K)
-        GGUFB200_G4_CASE(T_Q3_K)
-        GGUFB200_G4_CASE(T_Q4_K)
-        GGUFB200_G4_CASE(T_Q5_K)
-        GGUFB200_G4_CASE(T_Q6_K)
-        GGUFB200_G4_CASE(T_IQ4_NL)
-        GGUFB200_G4_CASE(T_IQ4_XS)
-    }
-#undef GGUFB200_G4_CASE
-    return GGUFB200_E_UNSUPPORTED;
+    const G4Args a{W, Wspan, span_stride, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, ws_bytes, flags, loraT, ldt, loraU, st};
+    return with_block(type, (int)GGUFB200_E_UNSUPPORTED, [&](auto q) {
+        using Q = decltype(q);
+        if (!Wspan && !packed_map_ok<Q>(W, K)) return (int)GGUFB200_E_UNSUPPORTED;
+        return with_act(act_dtype, [&](auto act) { return g4_run<Q, act.value>(a); });
+    });
 }
 
+// the canonical rows can be staged (every other weight needs the re-packed span-major layout of repack.cu)
 bool gemm4_supported(int type, const void *W, long long N, long long K)
 {
     if (N % 8 != 0 || K % 8 != 0) return false;
-    switch (type) {
-    case T_Q4_0: return g4_canonical_ok<Block<T_Q4_0>>(W, K);
-    case T_Q4_1: return g4_canonical_ok<Block<T_Q4_1>>(W, K);
-    case T_Q5_0: return g4_canonical_ok<Block<T_Q5_0>>(W, K);
-    case T_Q5_1: return g4_canonical_ok<Block<T_Q5_1>>(W, K);
-    case T_Q8_0: return g4_canonical_ok<Block<T_Q8_0>>(W, K);
-    case T_Q4_K: return g4_canonical_ok<Block<T_Q4_K>>(W, K);
-    case T_Q5_K: return g4_canonical_ok<Block<T_Q5_K>>(W, K);
-    case T_IQ4_NL: return g4_canonical_ok<Block<T_IQ4_NL>>(W, K);
-    }
-    return false;
+    return with_block(type, false, [&](auto q) { return packed_map_ok<decltype(q)>(W, K); });
 }
 
 }  // namespace ggufb200

@@ -224,44 +224,11 @@ static int gemv_launch(const void *W, long long N, long long K, const void *X, l
     return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
 }
 
-template <class Q, int MATH>
-static int gemv_act(const void *W, long long N, long long K, const void *X, long long M, long long ldx, int act, const void *bias, int bias_dtype,
-                    void *Y, long long ldy, cudaStream_t st)
-{
-    if (act == kBF16) return gemv_launch<Q, MATH, kBF16>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, st);
-    return gemv_launch<Q, MATH, kF16>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, st);
-}
-
-template <class Q>
-static int gemv_math(const void *W, long long N, long long K, const void *X, long long M, long long ldx, int act, int math, const void *bias,
-                     int bias_dtype, void *Y, long long ldy, cudaStream_t st)
-{
-    switch (math) {
-    case kF16: return gemv_act<Q, kF16>(W, N, K, X, M, ldx, act, bias, bias_dtype, Y, ldy, st);
-    case kBF16: return gemv_act<Q, kBF16>(W, N, K, X, M, ldx, act, bias, bias_dtype, Y, ldy, st);
-    case kF32: return gemv_act<Q, kF32>(W, N, K, X, M, ldx, act, bias, bias_dtype, Y, ldy, st);
-    }
-    return GGUFB200_E_DTYPE;
-}
-
 int gemv_dispatch(int type, const void *W, long long N, long long K, const void *X, long long M, long long ldx, int act_dtype, int math_dtype,
                   const void *bias, int bias_dtype, void *Y, long long ldy, cudaStream_t st)
 {
     if (M > kGemvMaxM) return GGUFB200_E_SHAPE;
-    switch (type) {
-    case T_Q4_0: return gemv_math<Block<T_Q4_0>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q4_1: return gemv_math<Block<T_Q4_1>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q5_0: return gemv_math<Block<T_Q5_0>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q5_1: return gemv_math<Block<T_Q5_1>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q8_0: return gemv_math<Block<T_Q8_0>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q2_K: return gemv_math<Block<T_Q2_K>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q3_K: return gemv_math<Block<T_Q3_K>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q4_K: return gemv_math<Block<T_Q4_K>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q5_K: return gemv_math<Block<T_Q5_K>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_Q6_K: return gemv_math<Block<T_Q6_K>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_IQ4_NL: return gemv_math<Block<T_IQ4_NL>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_IQ4_XS: return gemv_math<Block<T_IQ4_XS>>(W, N, K, X, M, ldx, act_dtype, math_dtype, bias, bias_dtype, Y, ldy, st);
-    case T_BF16: {
+    if (type == T_BF16) {
         const uint16_t *w = reinterpret_cast<const uint16_t *>(W);
         const uint8_t *x = reinterpret_cast<const uint8_t *>(X);
         uint8_t *y = reinterpret_cast<uint8_t *>(Y);
@@ -270,8 +237,13 @@ int gemv_dispatch(int type, const void *W, long long N, long long K, const void 
         else gemv_bf16w_kernel<kF16, 8><<<grid, kGemvThreads, 0, st>>>(w, N, K, x, ldx, (int)M, bias, bias_dtype, y, ldy);
         return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
     }
-    }
-    return GGUFB200_E_TYPE;
+    return with_block(type, (int)GGUFB200_E_TYPE, [&](auto q) {
+        return with_dtype(math_dtype, [&](auto math) {
+            return with_act(act_dtype, [&](auto act) {
+                return gemv_launch<decltype(q), math.value, act.value>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, st);
+            });
+        });
+    });
 }
 
 }  // namespace ggufb200

@@ -446,7 +446,7 @@ bool gemv2_supported(int type, const void *W, long long N, long long K, long lon
     if (type != T_Q4_K && type != T_Q5_K) return false;
     if (M < 1 || M > 8 || K % 256 != 0 || N < 1 || N > 0x7fffffffll / 16 || K > (1ll << 20)) return false;
     if ((reinterpret_cast<uintptr_t>(W) & 15) != 0) return false;          // tensor-map base; rows of whole 144 / 176-byte super-blocks are then 16-byte aligned
-    return type == T_Q4_K ? v2_plan<144>(N, K, M).ok : v2_plan<176>(N, K, M).ok;
+    return type == T_Q4_K ? v2_plan<Block<T_Q4_K>::TS>(N, K, M).ok : v2_plan<Block<T_Q5_K>::TS>(N, K, M).ok;
 }
 
 int gemv2_dispatch(int type, const void *W, long long N, long long K, const void *X, long long M, long long ldx, int act_dtype, const void *bias,
@@ -454,11 +454,10 @@ int gemv2_dispatch(int type, const void *W, long long N, long long K, const void
 {
     const int ws = w_stable ? 1 : 0;
     if (!gemv2_supported(type, W, N, K, M)) return GGUFB200_E_UNSUPPORTED;
-    if (type == T_Q4_K)
-        return act_dtype == kBF16 ? gemv2_launch<4, kBF16>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, st)
-                                  : gemv2_launch<4, kF16>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, st);
-    return act_dtype == kBF16 ? gemv2_launch<5, kBF16>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, st)
-                              : gemv2_launch<5, kF16>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, st);
+    return with_act(act_dtype, [&](auto act) {
+        return type == T_Q4_K ? gemv2_launch<4, act.value>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, st)
+                              : gemv2_launch<5, act.value>(W, N, K, X, M, ldx, bias, bias_dtype, Y, ldy, ws, st);
+    });
 }
 
 }  // namespace ggufb200

@@ -22,16 +22,6 @@
 
 namespace ggufb200 {
 
-template <class Q> struct SpanOf {
-    static constexpr int BYTES = (256 / Q::BS) * Q::TS;      // packed bytes of one row's 256-wide K-span
-    // Row pitch of a staged span in shared memory (and of the re-packed span-major layout, repack.cu).  A span whose byte
-    // count is a multiple of 16 keeps it (the canonical rows can then be staged by a 2-D tensor map, which writes rows
-    // densely); the others are padded to the next ODD multiple of 16: 16-byte aligned rows whose 16-byte reads at
-    // lane = row are bank-conflict free (Q2_K 84 -> 112, Q3_K 110 -> 112, IQ4_XS 136 -> 144, Q6_K 210 -> 240).
-    static constexpr int PAD16 = (BYTES + 15) / 16 * 16;
-    static constexpr int PITCH = BYTES % 16 == 0 ? BYTES : ((PAD16 / 16) % 2 == 1 ? PAD16 : PAD16 + 16);
-};
-
 // 16-byte / 4-byte loads of a staged span.  On the device the span always lives in shared memory (gemm4.cu): say so, or
 // the compiler emits generic loads (LD.E.128 + address-space resolution) instead of LDS.128.
 GG_HD uint4 ld_span16(const uint8_t *p)

@@ -13,7 +13,7 @@
 // The 128 rows of one CTA for one span are then 128*PITCH contiguous, 16-byte aligned bytes.  Pad bytes, rows >= N and the
 // tail of a ragged last span are zero (a zero block dequantises to 0 in every format).  The canonical bytes stay where
 // they are: GGMLTensor / state_dict semantics are untouched, the shadow is a cache the host layer may drop at any time.
-#include "produce.cuh"
+#include "blocks.cuh"
 
 namespace ggufb200 {
 
@@ -50,19 +50,11 @@ template <class Q> static int repack_run(const void *W, long long N, long long K
     return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
 }
 
-#define GGUFB200_REPACK_TYPES(X) \
-    X(T_Q4_0) X(T_Q4_1) X(T_Q5_0) X(T_Q5_1) X(T_Q8_0) X(T_Q2_K) X(T_Q3_K) X(T_Q4_K) X(T_Q5_K) X(T_Q6_K) X(T_IQ4_NL) X(T_IQ4_XS)
-
 // bytes of the shadow buffer and its geometry; 0 for types without a block layout
 size_t repack_bytes(int type, long long N, long long K, int *pitch, long long *span_stride)
 {
-    int pt = 0;
-    switch (type) {
-#define X(T) case T: pt = SpanOf<Block<T>>::PITCH; break;
-        GGUFB200_REPACK_TYPES(X)
-#undef X
-    default: return 0;
-    }
+    const int pt = with_block(type, 0, [](auto q) { return SpanOf<decltype(q)>::PITCH; });
+    if (pt == 0) return 0;
     const long long n_pad = (N + 255) / 256 * 256;
     if (pitch) *pitch = pt;
     if (span_stride) *span_stride = n_pad * pt;
@@ -71,12 +63,7 @@ size_t repack_bytes(int type, long long N, long long K, int *pitch, long long *s
 
 int repack_dispatch(int type, const void *W, long long N, long long K, void *out, cudaStream_t st)
 {
-    switch (type) {
-#define X(T) case T: return repack_run<Block<T>>(W, N, K, out, st);
-        GGUFB200_REPACK_TYPES(X)
-#undef X
-    }
-    return GGUFB200_E_TYPE;
+    return with_block(type, (int)GGUFB200_E_TYPE, [&](auto q) { return repack_run<decltype(q)>(W, N, K, out, st); });
 }
 
 }  // namespace ggufb200

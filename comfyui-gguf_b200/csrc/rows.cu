@@ -89,45 +89,10 @@ static int launch_rows(const void *packed, long long n_table_rows, long long K, 
     return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
 }
 
-template <class Q, int MATH>
-static int rows_out(const void *p, long long nt, long long K, const long long *rows, long long n, void *out, int od, cudaStream_t st)
-{
-    switch (od) {
-    case kF16: return launch_rows<Q, MATH, kF16>(p, nt, K, rows, n, out, st);
-    case kBF16: return launch_rows<Q, MATH, kBF16>(p, nt, K, rows, n, out, st);
-    case kF32: return launch_rows<Q, MATH, kF32>(p, nt, K, rows, n, out, st);
-    }
-    return GGUFB200_E_DTYPE;
-}
-
-template <class Q>
-static int rows_math(const void *p, long long nt, long long K, const long long *rows, long long n, void *out, int od, int md, cudaStream_t st)
-{
-    switch (md) {
-    case kF16: return rows_out<Q, kF16>(p, nt, K, rows, n, out, od, st);
-    case kBF16: return rows_out<Q, kBF16>(p, nt, K, rows, n, out, od, st);
-    case kF32: return rows_out<Q, kF32>(p, nt, K, rows, n, out, od, st);
-    }
-    return GGUFB200_E_DTYPE;
-}
-
 int rows_dispatch(int type, const void *packed, long long n_table_rows, long long K, const long long *rows, long long n_rows, void *out,
                   int out_dtype, int math_dtype, cudaStream_t st)
 {
-    switch (type) {
-    case T_Q4_0: return rows_math<Block<T_Q4_0>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q4_1: return rows_math<Block<T_Q4_1>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q5_0: return rows_math<Block<T_Q5_0>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q5_1: return rows_math<Block<T_Q5_1>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q8_0: return rows_math<Block<T_Q8_0>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q2_K: return rows_math<Block<T_Q2_K>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q3_K: return rows_math<Block<T_Q3_K>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q4_K: return rows_math<Block<T_Q4_K>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q5_K: return rows_math<Block<T_Q5_K>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_Q6_K: return rows_math<Block<T_Q6_K>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_IQ4_NL: return rows_math<Block<T_IQ4_NL>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_IQ4_XS: return rows_math<Block<T_IQ4_XS>>(packed, n_table_rows, K, rows, n_rows, out, out_dtype, math_dtype, st);
-    case T_BF16: {
+    if (type == T_BF16) {
         for (long long y0 = 0; y0 < n_rows; y0 += 65535) {
             long long ny = n_rows - y0 < 65535 ? n_rows - y0 : 65535;
             dim3 grid((unsigned)((K + kRowThreads * 4 - 1) / (kRowThreads * 4)), (unsigned)ny);
@@ -138,8 +103,13 @@ int rows_dispatch(int type, const void *packed, long long n_table_rows, long lon
         }
         return cudaGetLastError() == cudaSuccess ? GGUFB200_OK : GGUFB200_E_CUDA;
     }
-    }
-    return GGUFB200_E_TYPE;
+    return with_block(type, (int)GGUFB200_E_TYPE, [&](auto q) {
+        return with_dtype(math_dtype, [&](auto math) {
+            return with_dtype(out_dtype, [&](auto o) {
+                return launch_rows<decltype(q), math.value, o.value>(packed, n_table_rows, K, rows, n_rows, out, st);
+            });
+        });
+    });
 }
 
 }  // namespace ggufb200

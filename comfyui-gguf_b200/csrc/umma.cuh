@@ -1,5 +1,6 @@
-// umma.cuh -- PTX wrappers shared by the CTA-pair tensor-core kernels (gemm2.cu, gemm3.cu): cluster addressing,
-// cta_group::2 TMA / TMEM / tcgen05.mma / tcgen05.commit, TMEM loads, operand descriptors, epilogue helpers.
+// umma.cuh -- PTX wrappers of the CTA-pair tensor-core kernels (gemm2.cu, gemm3.cu, gemm4.cu): cluster addressing,
+// cta_group::2 TMA / TMEM / tcgen05.mma / tcgen05.commit, TMEM loads, operand descriptors, epilogue helpers; and the host
+// side's tensor-map encoders, which dequant.cu and gemv2.cu use as well.
 #pragma once
 #include <cuda.h>
 
@@ -184,5 +185,33 @@ static inline bool g2_make_map(CUtensorMap *tm, const void *base, long long rows
               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// Can make_packed_map stage the canonical rows of W: one row's span and the row stride multiples of 16 bytes, W 16-byte aligned
+template <class Q> static inline bool packed_map_ok(const void *W, long long K)
+{
+    const long long row_bytes = K / Q::BS * Q::TS;
+    return SpanOf<Q>::BYTES % 16 == 0 && row_bytes % 16 == 0 && (reinterpret_cast<uintptr_t>(W) & 15) == 0;
+}
+
+// 2-D tensor map over the raw packed rows of W [N rows, K / BS blocks]: one box = one row's span x 128 rows, no swizzle.  The inner
+// box extent is limited to 256 elements, so spans wider than 256 bytes use 2-byte elements (the kernels step the span coordinate
+// by SpanOf<Q>::BYTES / 2 then).
+template <class Q> static inline bool make_packed_map(CUtensorMap *tm, const void *W, long long N, long long K)
+{
+    constexpr int SPAN = SpanOf<Q>::BYTES;
+    G2EncodeFn fn = g2_encode_fn();
+    if (!fn) return false;
+    const long long row_bytes = K / Q::BS * Q::TS;
+    const bool wide = SPAN > 256;
+    cuuint64_t dims[2] = {(cuuint64_t)(wide ? row_bytes / 2 : row_bytes), (cuuint64_t)N};
+    cuuint64_t strides[1] = {(cuuint64_t)row_bytes};
+    cuuint32_t box[2] = {(cuuint32_t)(wide ? SPAN / 2 : SPAN), 128u};
+    cuuint32_t estr[2] = {1, 1};
+    return fn(tm, wide ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(W), dims, strides, box, estr,
+              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+// Split-K finalize of the fused kernels (gemm4.cu): Y[M, N] = act(sum of the fp32 slices P[splits][M][N] + bias), N % 8 == 0
+int splitk_finalize(const float *P, int splits, const void *bias, int bias_dtype, void *Y, long long M, long long N, long long ldy, int act_dtype,
+                    cudaStream_t st);
 
 }  // namespace ggufb200
